@@ -29,7 +29,12 @@ pass over the whole batch = one kernel launch per rank.
   gather (N>1)  the shards' rows gathered on GPU 0: fused evaluate+gather over NVLink peer memory against the NCCL
             gather, with a bit-identity flag.
 
---impl reference runs only the CPU arm (same config dict, bounded sample of the same rows) with "impl": "reference"."""
+--impl reference runs only the CPU arm (same config dict, bounded sample of the same rows) with "impl": "reference".
+
+--dump-outputs DIR writes what the last timed step left in HBM, for a fixed, seeded sample of the batch's trajectories
+(the same rows on any number of GPUs, at most 64 MB in all): DIR/F.npy [k, neF] and DIR/G.npy [k, neG], float64, the
+rows a caller of tolcuda_eval_batch receives.  The inputs depend only on the arguments, so two builds run with the
+same arguments can be compared output for output."""
 import argparse
 import json
 import os
@@ -53,6 +58,8 @@ WORKLOADS = {
     "G7_skywalker_ts100_B4096": ("G7_skywalker_ts100", 20260000, 4096),
 }
 RTOL, ATOL = 1e-12, 1e-14  # north_star tolerance
+DUMP_BYTES = 64 * 10**6 - 4096  # --dump-outputs: both .npy files together, headers included
+DUMP_SEED = 20261020
 
 
 def golden(name):
@@ -402,6 +409,31 @@ def time_launches(torch, ev, stream, X, outs, steps, overlap):
     return e0, e1
 
 
+def dump_outputs(directory, torch, dist, F, G, neF, neG, B_total, rank, world):
+    """--dump-outputs: rows of F and G (this rank's device buffers, rows = its shard) for a seeded sample of the global
+    trajectory indices, gathered on rank 0 and written as directory/F.npy and directory/G.npy"""
+    import tol_b200.synth as synth
+    k = min(B_total, DUMP_BYTES // (8 * (neF + neG)))
+    rows = np.sort(np.random.default_rng(DUMP_SEED).choice(B_total, k, replace=False))
+    b0, b1 = synth.shard_range(B_total, rank, world)
+    sel = np.flatnonzero((rows >= b0) & (rows < b1))
+    dev = F.device
+    src, dst = torch.from_numpy(rows[sel] - b0).to(dev), torch.from_numpy(sel).to(dev)
+    out = torch.zeros(k, neF + neG, dtype=torch.float64, device=dev)
+    out[dst, :neF] = F[src, :neF]
+    out[dst, neF:] = G[src, :neG]
+    if world > 1:  # every rank holds the sampled rows of its shard; take each row from its owner
+        parts = [torch.empty_like(out) for _ in range(world)]
+        dist.all_gather(parts, out)
+        owner = torch.from_numpy(rows // -(-B_total // world)).to(dev)
+        out = torch.stack(parts)[owner, torch.arange(k, device=dev)]
+    if rank == 0:
+        os.makedirs(directory, exist_ok=True)
+        out = out.cpu().numpy()
+        np.save(os.path.join(directory, "F.npy"), np.ascontiguousarray(out[:, :neF]))
+        np.save(os.path.join(directory, "G.npy"), np.ascontiguousarray(out[:, neF:]))
+
+
 def run_ours(args, wl_name):
     import torch
     import torch.distributed as dist
@@ -468,6 +500,9 @@ def run_ours(args, wl_name):
     ms_dev_local = e0.elapsed_time(e1)
     launches = ev.launches - l0
     clocks = sampler.stop(tw0, tw1)
+    if args.dump_outputs:  # before the serial loop below rewrites result set 0
+        F_, G_ = outs[(args.steps - 1) % len(outs)]
+        dump_outputs(args.dump_outputs, torch, dist, F_, G_, neF, neG, B_total, rank, world)
     # the same loop with plain launches (each waits for the previous grid's last CTA): secondary
     ser_steps = max(3, min(args.steps, 20))
     e0, e1 = time_launches(torch, ev, stream, Xd, outs[:1], ser_steps, 0)
@@ -881,7 +916,13 @@ def main():
     ap.add_argument("--gather-timeout", type=int, default=240)
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-ceiling", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write F and G of a seeded sample of the last timed step's rows as DIR/F.npy, DIR/G.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours: the reference arm keeps no output rows")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     if args.impl == "reference":
         run_reference_arm(args, args.workload)

@@ -96,6 +96,63 @@ def test_bench_reference_arm_prints_the_same_config_as_the_gpu_arm(oracle_built)
     assert r.returncode == 0 and r.stdout.strip() == ""
 
 
+def test_bench_dump_outputs_writes_a_fixed_sample_of_the_rows(tmp_path):
+    """bench.py --dump-outputs: the same seeded rows of F and G on every run, each row the caller's row of that
+    trajectory (padding left out), float64, the two files within 64 MB together; all rows when the batch fits"""
+    import sys
+    import torch
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    sys.path.insert(0, root)
+    import bench
+    neF, neG = 1612, 21437  # S10 ts = 200, the bench workload
+    for B in (400, 5):  # 347 rows of 400 fit the budget
+        F = torch.arange(B, dtype=torch.float64)[:, None] * 1e5 + torch.arange(neF + 3, dtype=torch.float64)
+        G = -torch.arange(B, dtype=torch.float64)[:, None] * 1e5 - torch.arange(neG + 5, dtype=torch.float64)
+        got = []
+        for run in range(2):
+            d = tmp_path / ("B%d_%d" % (B, run))
+            bench.dump_outputs(str(d), torch, None, F, G, neF, neG, B, 0, 1)
+            Fd, Gd = np.load(d / "F.npy"), np.load(d / "G.npy")
+            assert Fd.dtype == Gd.dtype == np.float64 and Fd.shape[1] == neF and Gd.shape[1] == neG
+            assert (d / "F.npy").stat().st_size + (d / "G.npy").stat().st_size <= 64 * 10**6
+            rows = (Fd[:, 0] / 1e5).astype(np.int64)
+            assert np.array_equal(Fd, F.numpy()[rows, :neF]) and np.array_equal(Gd, G.numpy()[rows, :neG])
+            got.append(rows)
+        assert np.array_equal(got[0], got[1]) and (np.diff(got[0]) > 0).all()
+        assert got[0].size == min(B, 347)
+
+
+def test_bench_dump_outputs_takes_each_row_from_the_rank_that_owns_it(tmp_path):
+    """bench.py --dump-outputs with the batch sharded over 3 ranks: each rank contributes the sampled rows of its own
+    shard, and rank 0 writes the same files one rank holding the whole batch writes"""
+    import sys
+    import torch
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    sys.path.insert(0, root)
+    import bench
+    import tol_b200.synth as synth
+    neF, neG, B, world = 1612, 21437, 1003, 3
+    F = torch.arange(B, dtype=torch.float64)[:, None] * 1e5 + torch.arange(neF, dtype=torch.float64)
+    G = -torch.arange(B, dtype=torch.float64)[:, None] * 1e5 - torch.arange(neG, dtype=torch.float64)
+    bench.dump_outputs(str(tmp_path / "one"), torch, None, F, G, neF, neG, B, 0, 1)
+    sent = {}
+
+    class Dist:  # all_gather of a stand-in process group: every rank's tensor, collected as the ranks call in
+        def __init__(self, rank):
+            self.rank = rank
+
+        def all_gather(self, parts, t):
+            sent[self.rank] = t.clone()
+            if len(sent) == world:
+                for q in range(world):
+                    parts[q].copy_(sent[q])
+    for rank in (2, 1, 0):  # rank 0, which writes, comes last so that its all_gather sees every shard
+        b0, b1 = synth.shard_range(B, rank, world)
+        bench.dump_outputs(str(tmp_path / "three"), torch, Dist(rank), F[b0:b1], G[b0:b1], neF, neG, B, rank, world)
+    for name in ("F.npy", "G.npy"):
+        assert np.array_equal(np.load(tmp_path / "three" / name), np.load(tmp_path / "one" / name))
+
+
 def test_bench_ceiling_is_the_slowest_resource():
     """bench.py's e2e lower bound (host side of the box): per path the slowest of PCIe in, DMA ingest and unavoidable
     host-DRAM traffic; the staging read-back only in the separate figure; full rows have no thread stores; a mix lies

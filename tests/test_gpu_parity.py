@@ -321,7 +321,7 @@ def test_full_size_properties(name, seed0, B, oracle_built):
     ev.close()
 
 
-def test_tolbatch_driver_end_to_end(tmp_path):
+def test_tolbatch_driver_end_to_end(tmp_path, param_root):
     """the C++ batch driver (reference CLI arguments + reference .param files -> initial guess ->
     perturbed batch -> all visible GPUs -> host gather): trajectory 0 is the reference's x0, so its
     objective must equal the reference's F[0]; every value finite; 2 runs agree bit for bit"""
@@ -330,11 +330,8 @@ def test_tolbatch_driver_end_to_end(tmp_path):
     import subprocess
     from conftest import ROOT
     exe = os.path.join(ROOT, "tol_b200", "tolbatch")
-    root = os.path.join(ROOT, "oracle", "_ref", "params")
-    if not os.path.isdir(root):
-        root = "/root/reference"
-    if not (os.path.exists(exe) and os.path.isdir(os.path.join(root, "aircraft"))):
-        pytest.skip("tolbatch or the reference .param files are not present")
+    root = param_root
+    assert os.path.exists(exe), "tolbatch is not built (make -C tol_b200/csrc)"
     for args, fixture in ((["0", "0", "70", "0", "-100", "0", "100", "tempest", "S10"], "S10_tempest_ts100"),
                           (["0", "0", "70", "400", "0", "0", "0", "skywalker", "G7"], "G7_skywalker_ts100")):
         g = load_golden(fixture)

@@ -56,12 +56,12 @@ def test_read_params_quirks(tmp_path):
         T.read_params(tmp_path / "missing.param")
 
 
-def test_read_params_matches_reference_files():
-    ref = "/root/reference/"
-    if not os.path.isdir(ref):
-        ref = os.path.join(ROOT, "oracle", "_ref", "params") + "/"
-    if not os.path.isdir(os.path.join(ref, "aircraft")):
-        pytest.skip("reference .param files not present")
+def test_read_params_matches_reference_files(param_root):
+    """tolcuda_read_params returns, with the reference's three degree -> radian conversions, the values the reference
+    read from its .param files (tests/golden/params.json): from its own files where oracle/_ref holds a copy, else from
+    files rebuilt from those values in the same layout (conftest.write_param_tree) -- then this checks the reader on
+    that layout (header comment, literal backslash-n, CRLF, degrees), not the reference's exact bytes"""
+    ref = param_root
     P = json.load(open(os.path.join(GOLDEN_DIR, "params.json")))
     for ac, want in P["aircraft"].items():
         v, cnt = T.read_params(os.path.join(ref, "aircraft", ac + ".param"))
@@ -410,16 +410,15 @@ def test_dump_writers_reject_misuse(tmp_path):
     assert L.tolcuda_set_dump_dir(None, b".") == -1
 
 
-def test_read_params_fuzz_against_the_reference_parser(tmp_path):
+def test_read_params_fuzz_against_the_reference_parser(tmp_path, param_root, pins):
     """tolcuda_read_params against the UNMODIFIED reference's parameters::readparams (src/parameters.cpp:14-34,
     reached through its `gain` constructor :77-94) on generated gains.param files: every line style std::stod
     accepts or rejects -- signs, exponents, hex floats, inf/nan, leading blanks, trailing text, CR, a literal
     backslash-n, a single '/' as the real delimiter, out-of-range literals and denormals (skipped), comment and
-    blank lines -- five accepted values per file, as the reference's size check wants (build container only)."""
+    blank lines -- five accepted values per file, as the reference's size check wants.  Against the compiled
+    reference where oracle/_ref is built, against its stored pins everywhere (conftest.Pins)."""
     import shutil
     import refclient as R
-    if not R.available():
-        pytest.skip("oracle/_ref (the compiled reference) is not present")
     rng = np.random.default_rng(20261018)
     accepted = ["{v!r}", "  \t{v!r}", "+{v!r}", "{v:.3e}", "{v:.17g}\\n   // gain", "{v!r}// c", "{v!r} / c", "{v!r}\r",
                 "{v!r}abc", "{v!r} 12", "{h}", "{v:.6f}/3", "{v:E}"]
@@ -428,7 +427,7 @@ def test_read_params_fuzz_against_the_reference_parser(tmp_path):
                 ". 5", "\t// x", "x0x10"]
     tmp = tmp_path / "root"
     for d in ("aircraft", "problems"):
-        shutil.copytree(os.path.join(R.REF_PARAMS, d), tmp / d)
+        shutil.copytree(os.path.join(param_root, d), tmp / d)
     gfile = tmp / "problems" / "S10" / "gains.param"
     os.chmod(gfile, 0o644)
     compared = 0
@@ -449,10 +448,15 @@ def test_read_params_fuzz_against_the_reference_parser(tmp_path):
             lines.append(rejected[int(rng.integers(len(rejected)))])
         text = "\n".join(lines) + ("\n" if trial % 2 else "")
         gfile.write_bytes(text.encode())
+        got, cnt = T.read_params(gfile)
+        # what the reference makes of the file: rejected (not five values), or these five values bit for bit
+        pins.check(np.array([cnt == 5]), got if cnt == 5 else np.zeros(0), what="trial %d: %r" % (trial, text))
+        if not R.available():
+            compared += cnt == 5
+            continue
         p = R.RefProblem.__new__(R.RefProblem)  # a problem object on the edited tree (no ts / gains rewriting)
         p._tmp = None
         p.h = R.lib().tolref_create(b"S10", b"tempest", 0.0, 0.0, 70.0, 0.0, -100.0, 0.0, 100.0, (str(tmp) + "/").encode())
-        got, cnt = T.read_params(gfile)
         if not p.h:  # the reference counted something other than five values ("+-3", "- 2", ...): so must the library
             assert cnt != 5, (text, got)
             continue
@@ -462,17 +466,16 @@ def test_read_params_fuzz_against_the_reference_parser(tmp_path):
         assert np.array_equal(got.view(np.int64), want.view(np.int64)), (text, got, want)  # bit for bit, NaN included
         compared += 1
     assert compared >= 30
+    pins.done()
 
 
-def test_setup_fuzz_against_the_reference(tmp_path):
+def test_setup_fuzz_against_the_reference(tmp_path, reference, pins):
     """tolcuda_problem_initial_guess / tolcuda_problem_bounds against the UNMODIFIED reference's InitialCond and
     setLimits (src/problemG7.cpp:19-217, src/problemS10.cpp:19-219, src/problem.cpp:198-365) on random command
     lines: both formulations, the five shipped aircraft, ts from 1 to 150, goals in every quadrant (and on the
     axes, where atan2 and the straight-line guess have their corner cases), loiter radii from 1 m to 1 km --
-    bit for bit, together with the closed-form dimensions and pattern (build container only)."""
-    import refclient as R
-    if not R.available():
-        pytest.skip("oracle/_ref (the compiled reference) is not present")
+    bit for bit, together with the closed-form dimensions and pattern.  Against the compiled reference where
+    oracle/_ref is built, against its stored pins everywhere (conftest.Pins)."""
     rng = np.random.default_rng(20261019)
     aircraft = ["skywalker", "tempest", "tempest_eric", "tempest_wences", "tempest_will"]
     goals = [(400.0, 0.0), (0.0, 400.0), (-250.0, 0.0), (0.0, -90.0), (1e-3, 1e-3)]
@@ -483,8 +486,9 @@ def test_setup_fuzz_against_the_reference(tmp_path):
         goal = (eg, ng, float(rng.uniform(-50, 120)), float(rng.choice([0.0, 1.0, 40.0, 100.0, 1000.0])))
         enu = (float(rng.uniform(-30, 30)), float(rng.uniform(-30, 30)), float(rng.uniform(0, 150)))
         ac = aircraft[trial % 5]
-        p = R.RefProblem(mission, ac, enu, goal, ts=ts)
+        p = reference(mission, ac, enu, goal, ts=ts)
         prm = p.params()
+        pins.check(prm["ac"], prm["gn"], prm["lm"], prm["sn"], prm["goal"], what="parameters of trial %d" % trial)
         lm = prm["lm"]
         cfg = T.make_config(mission, ts, prm["ac"], prm["gn"], prm["goal"],
                             limits=[lm[0], lm[1], lm[5], lm[2], lm[6], lm[3], lm[7], lm[4]], solver_tol=prm["sn"][4:6])
@@ -497,17 +501,17 @@ def test_setup_fuzz_against_the_reference(tmp_path):
         assert np.array_equal(x0.view(np.int64), rx0.view(np.int64)), (what, np.abs(x0 - rx0).max())
         for got, want, key in zip(T.bounds(cfg), p.bounds(), ("xlow", "xupp", "Flow", "Fupp")):
             assert np.array_equal(got.view(np.int64), want.view(np.int64)), (what, key)
+        pins.check(np.array(T.problem_dims(mission, ts)), i, j, x0, *T.bounds(cfg), what="setup of trial %d" % trial)
         p.close()
+    pins.done()
 
 
-def test_result_files_fuzz_against_the_reference(tmp_path):
+def test_result_files_fuzz_against_the_reference(tmp_path, reference, pins):
     """tolcuda_write_results_json / _txt against the UNMODIFIED reference's writeJSON / writeTXT
     (src/problem.cpp:1247-1418, jsoncpp's StyledWriter) on random states salted with the values number
     formatting trips over: +-0, integers, powers of ten, 0.1-like decimals, huge and tiny magnitudes,
-    denormals (build container only)"""
-    import refclient as R
-    if not R.available():
-        pytest.skip("oracle/_ref (the compiled reference) is not present")
+    denormals.  Against the compiled reference where oracle/_ref is built, against its stored pins everywhere
+    (conftest.Pins)."""
     rng = np.random.default_rng(20261022)
     salt = np.array([0.0, -0.0, 1.0, -1.0, 10.0, 100.0, 1e5, 1e15, 1e16, 1e17, 1e21, 1e22, -1e-5, 1e-4, 0.1, 0.2, 0.3,
                      1.0 / 3.0, 2.5, 123456789.0, 1e-300, 5e-324, 1.7976931348623157e308, 4.35, 0.5, 1e-7, 123.456,
@@ -519,7 +523,7 @@ def test_result_files_fuzz_against_the_reference(tmp_path):
         ac = aircraft[trial % 5]
         enu = tuple(float(v) for v in rng.choice([0.0, 70.0, -3.5, 12.25], 3))
         goal = tuple(float(v) for v in rng.uniform(-300, 300, 3)) + (float(rng.choice([0.0, 100.0, 33.3])),)
-        p = R.RefProblem(mission, ac, enu, goal, ts=ts)
+        p = reference(mission, ac, enu, goal, ts=ts)
         prm = p.params()
         lm = prm["lm"]
         cfg = T.make_config(mission, ts, prm["ac"], prm["gn"], prm["goal"],
@@ -537,19 +541,37 @@ def test_result_files_fuzz_against_the_reference(tmp_path):
         T.write_results_txt(cfg, x, F0, d / "ours.txt")
         assert (d / "ours.json").read_bytes() == (d / "ref.json").read_bytes(), (trial, mission, ts)
         assert (d / "ours.txt").read_bytes() == open(ref_txt, "rb").read(), (trial, mission, ts)
+        pins.check(x, (d / "ours.json").read_bytes(), (d / "ours.txt").read_bytes(), what="files of trial %d" % trial)
+    pins.done()
 
 
-def test_config_from_files_equals_what_the_reference_holds(tmp_path):
+def test_config_from_files_equals_what_the_reference_holds(tmp_path, param_root):
     """tolcuda_config_from_files (the file-reading half of tolcuda_create_from_files, host only) against the
     members of the UNMODIFIED reference's problem object built from the same files and command line
     (src/parameters.cpp:42-148, src/problem.cpp:13-60): aircraft with its degree -> radian conversions, gains,
-    limits, solver tolerances, ts, the ENU -> NED goal; and the errors of the reference's own checks"""
+    limits, solver tolerances, ts, the ENU -> NED goal; and the errors of the reference's own checks.  The members
+    are those the reference held for the command lines of tests/golden (stored there) and, where oracle/_ref is
+    built, those of live reference objects on random command lines."""
     import refclient as R
-    if not R.available():
-        pytest.skip("oracle/_ref (the compiled reference) is not present")
-    root = R.REF_PARAMS + "/"
+    root = param_root
+    P = json.load(open(os.path.join(GOLDEN_DIR, "params.json")))
+    for name in GOLDEN:
+        g = load_golden(name)
+        mission, ts = str(g["mission"]), int(g["ts"])
+        cfg = T.config_from_files(root, str(g["aircraft"]), mission, g["enu"], g["goal_enu"], ts=ts)
+        assert (cfg.formulation, cfg.ts, cfg.wind_model) == ({"G7": 7, "S10": 10}[mission], ts, 1), name
+        assert list(cfg.aircraft) == g["ac"].tolist(), name
+        assert list(cfg.gains) == P["problems"][mission]["gains"], name  # the *_gains fixtures edited gains.param
+        lm = g["lm"]
+        assert list(cfg.limits) == [lm[0], lm[1], lm[5], lm[2], lm[6], lm[3], lm[7], lm[4]], name
+        assert list(cfg.solver_tol) == g["sn"][4:6].tolist(), name
+        assert np.array_equal(np.array(list(cfg.goal)).view(np.int64), g["goal_ned"].view(np.int64)), name
+        assert np.array_equal(T.initial_guess(cfg).view(np.int64), g["x"][0].view(np.int64)), name
+        for got, key in zip(T.bounds(cfg), ("xlow", "xupp", "Flow", "Fupp")):
+            assert np.array_equal(got, g[key]), (name, key)
     rng = np.random.default_rng(5)
-    for trial, ac in enumerate(["skywalker", "tempest", "tempest_eric", "tempest_wences", "tempest_will"] * 2):
+    live = ["skywalker", "tempest", "tempest_eric", "tempest_wences", "tempest_will"] * 2 if R.available() else []
+    for trial, ac in enumerate(live):
         mission = "G7" if trial % 2 else "S10"
         enu = tuple(float(v) for v in rng.uniform(-50, 150, 3))
         goal = tuple(float(v) for v in rng.uniform(-400, 400, 4))
