@@ -280,6 +280,23 @@ int tolcuda_set_option(tolcuda_handle h, const char *name, long value);
 int tolcuda_eval_batch_summary(tolcuda_handle h, int B, const double *x, long ldx, double *F, long ldF,
                                double *G, long ldG, double *summary, long lds, int flags);
 
+/* Per-trajectory goals: one launch for trajectories of different missions (goal = the reference CLI's Eg Ng Ug Rg,
+ * src/arguments.cpp:32-46, which F and G depend on: S10's cost and objective row through r_k - rg, G7's boundary rows
+ * through chi_d = atan2(yg, xg) and dmax = |(xg, yg) - p_0|).  Aircraft, gains, ts and wind model stay the context's.
+ *   tolcuda_set_goals         keeps a goal table on the context's device: row b is goal[b*ldg + 0..3] = xg, yg, zg, rg
+ *                             in NED, as tolcuda_config.goal (ldg >= 4; host memory).  chi_d is derived per row on the
+ *                             host exactly as tolcuda_create derives it.  Synchronises the context's stream before it
+ *                             replaces the previous table, so TOLCUDA_NO_SYNC launches in flight finish with the table
+ *                             they were enqueued with.  count = 0 frees the table.
+ *   tolcuda_eval_batch_goals  as tolcuda_eval_batch_summary (summary may be NULL; every flag and option of it applies),
+ *                             but trajectory b of this call uses goal row row0 + b of the table.
+ * Row b of F, G and summary is bit for bit what a context created with row0 + b's goal (and the same options) writes
+ * for the same x.  No table, row0 < 0 or row0 + B > count (and a NULL handle) return TOLCUDA_EINVAL and launch nothing.
+ * The table lives in device memory: 64 bytes per row. */
+int tolcuda_set_goals(tolcuda_handle h, long count, const double *goal, long ldg);
+int tolcuda_eval_batch_goals(tolcuda_handle h, long row0, int B, const double *x, long ldx, double *F, long ldF,
+                             double *G, long ldG, double *summary, long lds, int flags);
+
 /* page-locked host memory for x/F/G of the host-pointer batch path (full PCIe speed, asynchronous
  * copies); plain wrappers so that a C/C++ driver needs no CUDA headers */
 int tolcuda_host_alloc(size_t bytes, void **ptr);

@@ -14,6 +14,8 @@
 #define TOLCUDA_PF 8       /* numstates, problems/<M>/snopt.param line 4 */
 #define TOLCUDA_REC 104    /* G values per collocation window: 8 defect rows x 13 columns */
 #define TOLCUDA_NVAR 31    /* of which depend on x (two more are -dt, the rest 0 or +-1) */
+/* doubles per row of a context's goal table (tolcuda_set_goals): xg, yg, rg, cos_chid, sin_chid, 3 unused; 64 bytes */
+#define TOLCUDA_GOAL_LD 8
 
 #ifdef __CUDACC__
 #define TOLCUDA_HD __host__ __device__

@@ -32,6 +32,8 @@ struct FgLaunch {
     int pdl;       // 0: ordinary launch; 1: programmatic dependent launch, the kernel waits for the preceding launch on
                    // the stream before its first store; 2: the same without the wait (outputs disjoint from the
                    // preceding launch's reads and writes).  Never set for op != 0 (d / lambda are read early).
+    const double *goals;  // NULL: every trajectory has the context's goal; else trajectory b's goal is the row
+                          // goals + TOLCUDA_GOAL_LD*b of a device goal table (op == 0 only)
     int sm_count;  // SMs of the device
     int device;    // CUDA device ordinal the launch goes to (the current device)
     cudaStream_t stream;

@@ -23,6 +23,11 @@
 //                                             written straight into GPU D's memory by the shards' own kernels
 //                                             (tolcuda_gather_*: NVLink peer stores, no host in between), timed, and
 //                                             compared bit for bit with the rows of the host gather
+//            [--goals FILE]                   one goal per trajectory: line b of FILE is `Eg Ng Ug Rg` (arguments 4-7 of
+//                                             the reference CLI) for trajectory b, whose initial guess is then the
+//                                             reference's for that goal; B = the line count (--batch, if given, must
+//                                             equal it).  One launch per device for all goals (tolcuda_eval_batch_goals);
+//                                             --results writes each trajectory's own goal.  Not with --gather-gpu.
 #include <chrono>
 #include <cctype>
 #include <cmath>
@@ -40,7 +45,8 @@ namespace {
 
 struct Args {
     double enu[3] = {0, 0, 0}, goal[4] = {0, 0, 0, 0};
-    std::string aircraft, mission, root = "./", xfile, json, results, host_path = "compact";
+    std::string aircraft, mission, root = "./", xfile, json, results, host_path = "compact", goals_file;
+    std::vector<double> goals;  // --goals: 4 per trajectory, xg, yg, zg, rg in NED (tolcuda_config.goal)
     int ts = 0, batch = 4096, gpus = 0, steps = 3, nresults = 4, gather_gpu = -1;
     bool summary_only = false;
     uint64_t seed = 1;
@@ -69,12 +75,43 @@ void check(int rc, const char *what) {
     if (rc) die(std::string(what) + " failed (" + std::to_string(rc) + "): " + tolcuda_last_error());
 }
 
+// --goals FILE: every line `Eg Ng Ug Rg` (ENU, radius), stored as the NED goal tolcuda_config_from_files makes of the
+// same command-line arguments (reference src/problem.cpp:24-27); anything else in the file is refused
+void read_goals(const std::string &path, std::vector<double> &out) {
+    FILE *f = std::fopen(path.c_str(), "r");
+    if (!f) die("cannot open goal file " + path);
+    std::string text;
+    char buf[4096];
+    for (size_t got; (got = std::fread(buf, 1, sizeof buf, f)) > 0;) text.append(buf, got);
+    std::fclose(f);
+    size_t pos = 0;
+    for (long line = 1; pos < text.size(); line++) {
+        size_t end = text.find('\n', pos);
+        if (end == std::string::npos) end = text.size();
+        const std::string ln = text.substr(pos, end - pos);
+        pos = end + 1;
+        double v[4];
+        const char *p = ln.c_str();
+        for (int i = 0; i < 4; i++) {
+            char *q;
+            v[i] = std::strtod(p, &q);
+            if (q == p || !std::isfinite(v[i])) die(path + ":" + std::to_string(line) + ": want `Eg Ng Ug Rg`");
+            p = q;
+        }
+        while (std::isspace((unsigned char)*p)) p++;
+        if (*p) die(path + ":" + std::to_string(line) + ": want `Eg Ng Ug Rg`, found more");
+        out.insert(out.end(), {v[1], v[0], -v[2], v[3]});
+    }
+    if (out.empty()) die(path + ": no goals");
+}
+
 Args parse(int argc, char **argv) {
     if (argc < 10)
         die("usage: tolbatch E N U Eg Ng Ug Rg aircraft mission [--root DIR/] [--ts N] [--batch B] [--gpus G] "
             "[--seed S] [--perturb REL,ABS] [--x-file F] [--steps K] [--json OUT] [--results DIR [--nresults K]] [--summary-only] "
-            "[--gather-gpu D]");
+            "[--gather-gpu D] [--goals FILE]");
     Args a;
+    bool batch_set = false;
     for (int i = 0; i < 3; i++) a.enu[i] = std::atof(argv[1 + i]);  // as src/arguments.cpp:35-41 (atof)
     for (int i = 0; i < 4; i++) a.goal[i] = std::atof(argv[4 + i]);
     a.aircraft = argv[8];
@@ -87,7 +124,8 @@ Args parse(int argc, char **argv) {
         };
         if (k == "--root") a.root = val();
         else if (k == "--ts") a.ts = std::atoi(val());
-        else if (k == "--batch") a.batch = std::atoi(val());
+        else if (k == "--batch") a.batch = std::atoi(val()), batch_set = true;
+        else if (k == "--goals") a.goals_file = val();
         else if (k == "--gpus") a.gpus = std::atoi(val());
         else if (k == "--steps") a.steps = std::atoi(val());
         else if (k == "--seed") a.seed = std::strtoull(val(), nullptr, 10);
@@ -112,6 +150,14 @@ Args parse(int argc, char **argv) {
         !(std::isdigit((unsigned char)a.host_path[0]) && std::atoi(a.host_path.c_str()) <= 100))
         die("--host-path wants compact, full, auto or a percentage 0..100");
     if (a.gather_gpu >= 0 && a.summary_only) die("--gather-gpu gathers F and G rows: not available with --summary-only");
+    if (!a.goals_file.empty()) {
+        if (a.gather_gpu >= 0) die("--goals cannot be combined with --gather-gpu (the gather protocol has no goal table)");
+        read_goals(a.goals_file, a.goals);
+        const long lines = (long)a.goals.size() / 4;
+        if (batch_set && lines != a.batch)
+            die(a.goals_file + ": " + std::to_string(lines) + " goals for --batch " + std::to_string(a.batch));
+        a.batch = (int)lines;
+    }
     return a;
 }
 
@@ -160,14 +206,27 @@ int main(int argc, char **argv) {
         for (int b = 0; b < B; b++) {
             Rng r(a.seed * 0x100000001b3ULL + (uint64_t)b);
             double *xb = X + (size_t)b * ldx;
+            if (!a.goals.empty()) {  // the reference's initial guess for this trajectory's goal (G7's rotates by chi_d)
+                tolcuda_config cb = cfg;
+                for (int i = 0; i < 4; i++) cb.goal[i] = a.goals[4 * (size_t)b + i];
+                check(tolcuda_problem_initial_guess(&cb, x0.data()), "initial guess");
+            }
+            // with --goals and --perturb 0,0 every row is its goal's x0 itself (x0 + 0*u would turn -0.0 into +0.0), so
+            // its result file is the one a single-goal run writes for trajectory 0
+            const bool copy = b == 0 || (!a.goals.empty() && a.rel == 0.0 && a.abs_ == 0.0);
             for (int i = 0; i < n; i++) {
                 const double u = r.sym(), up = r.sym();
-                xb[i] = b == 0 ? x0[i] : x0[i] * (1.0 + a.rel * u) + a.abs_ * up;  // trajectory 0 is x0 itself
+                xb[i] = copy ? x0[i] : x0[i] * (1.0 + a.rel * u) + a.abs_ * up;  // trajectory 0 is x0 itself
             }
         }
     }
 
     // evaluate: one host thread per device, contiguous block of trajectory indices each, no collective
+    const int per_dev = (B + G - 1) / G;
+    for (int g = 0; g < G && !a.goals.empty(); g++) {  // each device's context holds its shard's rows of the goal table
+        const int b0 = std::min(B, g * per_dev), b1 = std::min(B, b0 + per_dev);
+        check(tolcuda_set_goals(h[g], b1 - b0, a.goals.data() + 4 * (size_t)b0, 4), "tolcuda_set_goals");
+    }
     std::vector<double> secs(G, 0.0);
     double best = 1e300;
     // share of the chunks that cross PCIe as full rows (tolcuda_set_option "full_rows_pct"; 100 = all of them)
@@ -204,9 +263,17 @@ int main(int argc, char **argv) {
         const auto t0 = std::chrono::steady_clock::now();
         for (int g = 0; g < G; g++)
             th.emplace_back([&, g]() {
-                const int per = (B + G - 1) / G, b0 = std::min(B, g * per), b1 = std::min(B, b0 + per);
+                const int b0 = std::min(B, g * per_dev), b1 = std::min(B, b0 + per_dev);
                 const auto s0 = std::chrono::steady_clock::now();
-                if (b1 > b0 && a.summary_only)
+                if (b1 > b0 && !a.goals.empty())
+                    check(a.summary_only
+                              ? tolcuda_eval_batch_goals(h[g], 0, b1 - b0, X + (size_t)b0 * ldx, ldx, nullptr, 0, nullptr, 0,
+                                                         S + (size_t)b0 * 4, 4, TOLCUDA_HOST_PTRS)
+                              : tolcuda_eval_batch_goals(h[g], 0, b1 - b0, X + (size_t)b0 * ldx, ldx, F + (size_t)b0 * ldF,
+                                                         ldF, Gv + (size_t)b0 * ldG, ldG, nullptr, 0,
+                                                         TOLCUDA_NEED_F | TOLCUDA_NEED_G | TOLCUDA_HOST_PTRS),
+                          "tolcuda_eval_batch_goals");
+                else if (b1 > b0 && a.summary_only)
                     check(tolcuda_eval_batch_summary(h[g], b1 - b0, X + (size_t)b0 * ldx, ldx, nullptr, 0, nullptr, 0,
                                                      S + (size_t)b0 * 4, 4, TOLCUDA_HOST_PTRS),
                           "tolcuda_eval_batch_summary");
@@ -324,7 +391,9 @@ int main(int argc, char **argv) {
     if (!a.results.empty())
         for (int b = 0; b < std::min(B, a.nresults); b++) {
             const std::string path = a.results + "/snopt_results_" + std::to_string(b) + ".json";
-            check(tolcuda_write_results_json(&cfg, a.aircraft.c_str(), a.mission.c_str(), a.enu[0], a.enu[1], a.enu[2],
+            tolcuda_config cb = cfg;  // "args" holds the trajectory's own goal
+            for (int i = 0; i < 4 && !a.goals.empty(); i++) cb.goal[i] = a.goals[4 * (size_t)b + i];
+            check(tolcuda_write_results_json(&cb, a.aircraft.c_str(), a.mission.c_str(), a.enu[0], a.enu[1], a.enu[2],
                                              X + (size_t)b * ldx, obj[b], path.c_str()),
                   "tolcuda_write_results_json");
         }

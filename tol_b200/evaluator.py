@@ -365,6 +365,37 @@ class Evaluator:
             G.ctypes.data if needG else None, self.neG, S.ctypes.data, 4, flags))
         return S, F, G
 
+    def set_goals(self, goals_ned):
+        """tolcuda_set_goals: the context's goal table, one row (xg, yg, zg, rg in NED) per trajectory of
+        eval_batch_goals; an empty array frees it"""
+        g = np.ascontiguousarray(goals_ned, dtype=np.float64).reshape(-1, 4)
+        _l.check(self.L.tolcuda_set_goals(self.h, g.shape[0], g.ctypes.data if g.size else None, 4))
+
+    def eval_batch_goals(self, X, F=None, G=None, row0=0, summary=None, needF=True, needG=True, sync=True,
+                         compact_rows=False, full_copy=False, overlap=0):
+        """tolcuda_eval_batch_goals: row b of X with goal row row0 + b of the table (set_goals).  X, F, G, summary are
+        numpy arrays (host path; F, G allocated if None and asked for) or torch CUDA tensors (device path, like
+        eval_batch_device: sync / overlap apply there).  summary: [B, >= 4] or None.  Returns F, G, summary."""
+        B = X.shape[0]
+        dev = hasattr(X, "data_ptr")
+        if dev:
+            self._follow_torch(X)
+            ptr, ld = (lambda a: a.data_ptr() if a is not None else None), (lambda a: a.stride(0) if a is not None else 0)
+            flags = DEVICE_PTRS | (0 if sync else NO_SYNC)
+            flags |= (OVERLAP if overlap == 1 else 0) | (OVERLAP_DISJOINT if overlap == 2 else 0)
+        else:
+            assert X.dtype == np.float64 and X.strides[1] == 8
+            if F is None and needF:
+                F = np.empty((B, self.neF))
+            if G is None and needG:
+                G = np.empty((B, self.compact_len if compact_rows else self.neG))
+            ptr, ld = (lambda a: a.ctypes.data if a is not None else None), (lambda a: a.strides[0] // 8 if a is not None else 0)
+            flags = HOST_PTRS | (FULL_G_COPY if full_copy else 0)
+        flags |= (NEED_F if needF else 0) | (NEED_G if needG else 0) | (COMPACT_G if compact_rows else 0)
+        _l.check(self.L.tolcuda_eval_batch_goals(self.h, int(row0), B, ptr(X), ld(X), ptr(F), ld(F), ptr(G), ld(G),
+                                                 ptr(summary), ld(summary), flags))
+        return F, G, summary
+
     def stream_signal(self, flag_ptr, value):
         """tolcuda_stream_signal: *flag = value after everything enqueued so far on the context's stream"""
         _l.check(self.L.tolcuda_stream_signal(self.h, C.c_void_p(flag_ptr), int(value) & 0xffffffff))

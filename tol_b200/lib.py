@@ -52,6 +52,9 @@ def load():
     L.tolcuda_eval.argtypes = [vp, dp, C.c_int, dp, C.c_int, dp]
     L.tolcuda_eval_batch.argtypes = [vp, C.c_int, vp, C.c_long, vp, C.c_long, vp, C.c_long, C.c_int]
     L.tolcuda_eval_batch_summary.argtypes = [vp, C.c_int, vp, C.c_long, vp, C.c_long, vp, C.c_long, vp, C.c_long, C.c_int]
+    L.tolcuda_set_goals.argtypes = [vp, C.c_long, vp, C.c_long]
+    L.tolcuda_eval_batch_goals.argtypes = [vp, C.c_long, C.c_int, vp, C.c_long, vp, C.c_long, vp, C.c_long, vp, C.c_long,
+                                           C.c_int]
     L.tolcuda_compact_len.argtypes = [C.c_int, C.c_int]
     L.tolcuda_compact_len.restype = C.c_long
     L.tolcuda_expand_compact_g.argtypes = [C.c_int, C.c_int, C.c_long, vp, C.c_long, vp, C.c_long, C.c_int]

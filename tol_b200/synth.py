@@ -23,6 +23,27 @@ def batch(x0, seed0, b0, b1, out=None, ld=None):
     return out
 
 
+SEED_GOALS = 20280000
+
+
+def goals(mission, lo, hi, seed=SEED_GOALS):
+    """goals (xg, yg, zg, rg in NED) of trajectories lo..hi-1 of a batch with per-trajectory goals, [hi-lo, 4].  Row b
+    comes from numpy.random.Generator(PCG64(seed + b)) alone, so any sharding of the batch gives the same table.
+    The goal lies 300..3000 m from the origin (where the reference puts the aircraft's initial position) at 50..150 m
+    altitude, S10 loiter radii 50..400 m.  G7 (whose boundary rows depend on chi_d = atan2(yg, xg)): the even rows sit
+    within 1e-9 rad of the +x, +y, -x, -y axis in turn (b mod 8 = 0, 2, 4, 6; the -x axis on both sides of the branch
+    cut of atan2), the odd rows at uniform bearings, so the table covers all four quadrants of chi_d and each axis."""
+    out = np.empty((hi - lo, 4))
+    for b in range(lo, hi):
+        r = np.random.Generator(np.random.PCG64(seed + b)).uniform(0.0, 1.0, size=5)
+        chi = -np.pi + 2.0 * np.pi * r[0]
+        if mission in ("G7", 7) and b % 2 == 0:
+            chi = (b % 8) // 2 * (np.pi / 2) + (r[0] - 0.5) * 2e-9
+        dist = 300.0 + 2700.0 * r[1]
+        out[b - lo] = (dist * np.cos(chi), dist * np.sin(chi), -(50.0 + 100.0 * r[2]), 50.0 + 350.0 * r[3])
+    return out
+
+
 def shard_range(B, rank, world):
     """contiguous block of trajectory indices owned by `rank` (SURVEY.md section 8e)"""
     per = (B + world - 1) // world
