@@ -241,6 +241,24 @@ int tolcuda_jac_vec(tolcuda_handle h, int B, const double *x, long ldx, const do
                     int flags);
 int tolcuda_jac_tvec(tolcuda_handle h, int B, const double *x, long ldx, const double *lambda, long ldl, double *z,
                      long ldz, int flags);
+/* Hessian of the Lagrangian times a vector (a truncated-Newton / trust-region CG step or an exact-Hessian SQP step on
+ * the GPU), with J as above:
+ *   w_b = D_x[ J(x_b)^T lambda_b ] d_b,   w[b*ldw + j] = sum_i lambda_i sum_l (dJ_ij / dx_l) d_l
+ * x: n per row, lambda: neF (lambda[0] weights the objective row, IPOPT's sigma), d: n, w: n.  z, if not NULL,
+ * receives J(x_b)^T lambda_b (n per row) bit for bit as tolcuda_jac_tvec writes it.  Where G is the gradient of F this
+ * is the Hessian of lambda^T F times d.  G7's objective row is the gradient of 1/2 kT sum T^2 + kp ts dt / dist (kp
+ * where F[0] uses kv, as in the reference), its boundary row 11 that of dist alone (the reference leaves out the
+ * node-0 derivative of dmax); w differentiates those rows.  S10's boundary-row dt entries are the constant 0.  G holds
+ * the wind and its gradient fixed while its entries depend on them, and w differentiates the entries with the wind
+ * included: the operator is symmetric under wind model 0, not under models 1 and 3 (DESIGN.md 5).  The kernels evaluate every window's Jacobian entries in forward-mode dual arithmetic and
+ * consume them in registers, moving 8*(3n + neF) bytes per trajectory (+ 8n with z).
+ * Device pointers on the context's device; flags: 0 or TOLCUDA_NO_SYNC (TOLCUDA_HOST_PTRS: TOLCUDA_EUNSUPPORTED).  A
+ * null x, lambda, d or w, or a leading dimension shorter than its row, is TOLCUDA_EINVAL; B = 0 launches nothing.
+ * Evaluated with the context's goal; the options "kernel", "per", "lwarps" and "per_min_waves" apply as to
+ * tolcuda_jac_tvec, and every option gives the same bits except w[0] and z[0] (sums over the trajectory) under
+ * kernel L. */
+int tolcuda_lag_hess_vec(tolcuda_handle h, int B, const double *x, long ldx, const double *lambda, long ldl,
+                         const double *d, long ldd, double *w, long ldw, double *z, long ldz, int flags);
 /* host threads the host-pointer batch path of this context expands compact rows with (0 = default:
  * environment TOLCUDA_HOST_THREADS, else the cores available to the process / LOCAL_WORLD_SIZE) */
 int tolcuda_set_host_threads(tolcuda_handle h, int threads);

@@ -21,7 +21,12 @@ struct FgLaunch {
     int needF, needG;
     double *S;  // optional per-trajectory summary [B][ldS >= 4]: objective, max|defect|, max|boundary|, sum defect^2
     long ldS;
-    int op;  // 0: F/G; 1: y = J d (F receives y [neF], G holds d [n]); 2: z = J^T lambda (F holds lambda [neF], G receives z [n])
+    int op;  // 0: F/G; 1: y = J d (F receives y [neF], G holds d [n]); 2: z = J^T lambda (F holds lambda [neF], G receives z [n]);
+             // 3: w = D_x[J^T lambda] d (F holds lambda [neF], G receives w [n], D holds d [n], Z receives z [n] or is NULL)
+    const double *D;  // op 3: d
+    long ldD;
+    double *Z;        // op 3: z = J^T lambda, optional
+    long ldZ;
     int compact;  // G/ldG address the compact layout [R0 | 31 per window | boundary block] (host-pointer path)
     int kernel;    // 0/1 = kernel A (CTA per run of trajectories), 2 = kernel L (CTA per trajectory, tile loop; any ts)
     int lwarps;    // kernel L: warps per CTA (0: the count that balances the tiles)

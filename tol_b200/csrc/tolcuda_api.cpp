@@ -119,9 +119,11 @@ void goal_row(const double *goal, double row[TOLCUDA_GOAL_LD]) {
 // goals: NULL, or the device goal-table row of the launch's first trajectory
 int launch(tolcuda_ctx *h, cudaStream_t st, int B, const double *x, long ldx, double *F, long ldF,
            double *G, long ldG, int needF, int needG, double *S = nullptr, long ldS = 0, int compact = 0, int op = 0,
-           int pdl = 0, const double *goals = nullptr) {
+           int pdl = 0, const double *goals = nullptr, const double *D = nullptr, long ldD = 0, double *Z = nullptr,
+           long ldZ = 0) {
     FgLaunch L{};
     L.goals = goals;
+    L.D = D, L.ldD = ldD, L.Z = Z, L.ldZ = ldZ;
     L.S = S, L.ldS = ldS;
     L.compact = compact;
     L.op = op;
@@ -896,6 +898,28 @@ int tolcuda_jac_vec(tolcuda_handle h, int B, const double *x, long ldx, const do
 int tolcuda_jac_tvec(tolcuda_handle h, int B, const double *x, long ldx, const double *lambda, long ldl, double *z,
                      long ldz, int flags) {
     return jac_op(h, 2, B, x, ldx, lambda, ldl, h ? h->c.neF : 0, z, ldz, h ? h->c.n : 0, flags, "tolcuda_jac_tvec");
+}
+
+// w = D_x[J(x)^T lambda] d and optionally z = J(x)^T lambda (fg_kernels.cu, MODE_HVP)
+int tolcuda_lag_hess_vec(tolcuda_handle h, int B, const double *x, long ldx, const double *lambda, long ldl,
+                         const double *d, long ldd, double *w, long ldw, double *z, long ldz, int flags) {
+    if (!h || B < 0) return TOLCUDA_EINVAL;
+    if (B == 0) return 0;
+    const FgConst &c = h->c;
+    if (!x || !lambda || !d || !w || ldx < c.n || ldl < c.neF || ldd < c.n || ldw < c.n || (z && ldz < c.n)) {
+        set_error("tolcuda_lag_hess_vec: null pointer or leading dimension shorter than the row");
+        return TOLCUDA_EINVAL;
+    }
+    if (flags & TOLCUDA_HOST_PTRS) {
+        set_error("tolcuda_lag_hess_vec: device pointers only");
+        return TOLCUDA_EUNSUPPORTED;
+    }
+    CU(cudaSetDevice(h->cfg.device));
+    int rc = launch(h, h->stream, B, x, ldx, const_cast<double *>(lambda), ldl, w, ldw, 1, 1, nullptr, 0, 0, 3, 0, nullptr,
+                    d, ldd, z, z ? ldz : 0);
+    if (rc) return rc;
+    if (!(flags & TOLCUDA_NO_SYNC)) CU(cudaStreamSynchronize(h->stream));
+    return 0;
 }
 
 int tolcuda_problem_pattern_csc(int formulation, int ts, int *colptr, int *rowidx, int *perm) {

@@ -352,6 +352,16 @@ class Evaluator:
         _l.check(self.L.tolcuda_jac_tvec(self.h, X.shape[0], X.data_ptr(), X.stride(0), Lam.data_ptr(), Lam.stride(0),
                                          Z.data_ptr(), Z.stride(0), 0 if sync else NO_SYNC))
 
+    def lag_hess_vec(self, X, Lam, D, W, Z=None, sync=True):
+        """tolcuda_lag_hess_vec: W[b] = D_x[J(X[b])^T Lam[b]] D[b], the Hessian of the Lagrangian Lam[b]^T F times D[b],
+        and, if Z is given, Z[b] = J(X[b])^T Lam[b] (torch CUDA tensors [B, >= n], [B, >= neF], [B, >= n], [B, >= n],
+        [B, >= n])"""
+        self._follow_torch(X)
+        _l.check(self.L.tolcuda_lag_hess_vec(self.h, X.shape[0], X.data_ptr(), X.stride(0), Lam.data_ptr(), Lam.stride(0),
+                                             D.data_ptr(), D.stride(0), W.data_ptr(), W.stride(0),
+                                             None if Z is None else Z.data_ptr(), 0 if Z is None else Z.stride(0),
+                                             0 if sync else NO_SYNC))
+
     def summary_host(self, X, needF=False, needG=False):
         """tolcuda_eval_batch_summary with host arrays: [B, 4] = objective, max|defect|, max boundary
         violation, sum defect^2 (F and G are not produced unless asked for)"""

@@ -6,7 +6,9 @@ build's ptxas logs and SASS mnemonic counts from `cuobjdump -sass tol_b200/libto
 
 Template arguments of fg_cta_kernel<FORM, WIND, MAXT, PER, MODE, LOOP> / fg_long_kernel<FORM, WIND, MODE>:
 FORM 7 = G7, 10 = S10; WIND 0 / 1 / 3; MODE 0 PLAIN, 1 SUMMARY, 2 COMPACT, 3 JVP, 4 VJP, 5 F only, 6 F only + summary
-(fg_kernels.cu); fg_cta_goals_kernel / fg_long_goals_kernel are the same instances with a per-trajectory goal table."""
+(fg_kernels.cu); fg_cta_goals_kernel / fg_long_goals_kernel are the same instances with a per-trajectory goal table;
+fg_cta_hvp_kernel<FORM, WIND, MAXT, PER, LOOP> / fg_long_hvp_kernel<FORM, WIND> are MODE 7, the Hessian-of-the-Lagrangian
+product (dual arithmetic)."""
 import collections
 import os
 import re
