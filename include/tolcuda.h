@@ -293,6 +293,10 @@ int tolcuda_set_option(tolcuda_handle h, const char *name, long value);
  *   summary[b*lds + 1] = max |defect|              over the 8*ts dynamics rows
  *   summary[b*lds + 2] = max boundary violation    |row| for equality rows, max(row, 0) for G7's dist <= dmax
  *   summary[b*lds + 3] = sum of defect^2
+ * Non-finite rows: the maxima are NaN when any of their rows is NaN (a NaN defect or boundary row is not hidden by
+ * finite ones), +inf when a row is +-inf and none is NaN; the sum is NaN or +inf likewise.  Each entry is what
+ * numpy's max / sum give on the F this call writes, so screening on summary[b*lds + 1] < tol rejects a trajectory
+ * whose defects are NaN.
  * lds >= 4; same pointer kind as x/F/G.  With neither TOLCUDA_NEED_F nor TOLCUDA_NEED_G only the summary
  * is produced (F and G may then be NULL). */
 int tolcuda_eval_batch_summary(tolcuda_handle h, int B, const double *x, long ldx, double *F, long ldF,

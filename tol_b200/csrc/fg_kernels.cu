@@ -194,9 +194,13 @@ struct TileSums {
     double dmax, dssq;  // max |defect|, sum of defect^2 (SUMM instantiations only)
 };
 
+// the larger of a and b, NaN if either is NaN (fmax drops a NaN operand): a summary maximum over values one of which is
+// NaN is NaN, as numpy's max of the same values, so a NaN defect or boundary row cannot hide behind finite ones
+__device__ __forceinline__ double max_nan(double a, double b) { return (a > b || a != a) ? a : b; }
+
 __device__ __forceinline__ double warp_max(double v) {
 #pragma unroll
-    for (int m = 16; m > 0; m >>= 1) v = fmax(v, __shfl_xor_sync(0xffffffffu, v, m));
+    for (int m = 16; m > 0; m >>= 1) v = max_nan(v, __shfl_xor_sync(0xffffffffu, v, m));
     return v;
 }
 
@@ -776,7 +780,7 @@ __device__ __forceinline__ void tile_eval(const FgConst &c, double *sx, double *
         if (active) {
 #pragma unroll
             for (int i = 0; i < PF; i++) {
-                m = fmax(m, fabs(f[i]));
+                m = max_nan(m, fabs(f[i]));
                 q += f[i] * f[i];
             }
         }
@@ -1095,7 +1099,7 @@ __device__ __forceinline__ void traj_epilogue(const FgConst &c, const GoalT gl, 
             if (lane >= 2 && lane < PX) bval = ne - n0;
             if (lane == 0) bval = ddx - dist * gl.cos_chid(c);
             if (lane == 1) bval = ddy - dist * gl.sin_chid(c);
-            if (lane == PX) bval = fmax(dist - sqrt(gx * gx + gy * gy), 0.0);  // dist <= dmax: only excess counts
+            if (lane == PX) bval = max_nan(dist - sqrt(gx * gx + gy * gy), 0.0);  // dist <= dmax: only excess counts
         }
         if (needG && lane == 0) {
             // objective row ends, src/problemG7.cpp:343-380 (sic: kp, where cost() uses kv)
@@ -1393,7 +1397,7 @@ __device__ __forceinline__ void fg_cta_body(const FgConst &c, int nrun, int per_
                 tT += vred[w];
                 tp += vred[32 + w];
                 if (SUMM) {
-                    dmax = fmax(dmax, vred[64 + w]);
+                    dmax = max_nan(dmax, vred[64 + w]);
                     dssq += vred[96 + w];
                 }
             }
@@ -1513,7 +1517,7 @@ __device__ __forceinline__ void fg_long_body(const FgConst &c, const double *__r
         __syncwarp();
         accT += tsum.sumT;
         accp += tsum.sump;
-        accm = fmax(accm, tsum.dmax);
+        accm = max_nan(accm, tsum.dmax);
         accq += tsum.dssq;
         slot ^= 1;
     }
@@ -1541,7 +1545,7 @@ __device__ __forceinline__ void fg_long_body(const FgConst &c, const double *__r
         tT += vred[w];
         tp += vred[32 + w];
         if (SUMM) {
-            dmax = fmax(dmax, vred[64 + w]);
+            dmax = max_nan(dmax, vred[64 + w]);
             dssq += vred[96 + w];
         }
     }

@@ -309,8 +309,10 @@ int main(int argc, char **argv) {
     for (int b = 0; b < B && !a.summary_only; b++) {
         const double *Fb = F + (size_t)b * ldF, *Gb = Gv + (size_t)b * ldG;
         double d = 0.0, e = 0.0;
-        for (int i = 1; i < neF - nb; i++) d = std::fmax(d, std::fabs(Fb[i]));
-        for (int i = neF - nb; i < neF; i++) e = std::fmax(e, std::fabs(Fb[i]));
+        // NaN if a row is NaN, as the summary's maxima (tolcuda.h): std::fmax would drop it
+        const auto max_nan = [](double u, double v) { return (u > v || u != u) ? u : v; };
+        for (int i = 1; i < neF - nb; i++) d = max_nan(d, std::fabs(Fb[i]));
+        for (int i = neF - nb; i < neF; i++) e = max_nan(e, std::fabs(Fb[i]));
         for (int i = 0; i < neF; i++) nonfinite += !std::isfinite(Fb[i]);
         for (int i = 0; i < neG; i++) nonfinite += !std::isfinite(Gb[i]);
         obj[b] = Fb[0], defect[b] = d, bnd[b] = e;
