@@ -789,7 +789,7 @@ def test_api_misuse_is_reported_not_executed():
     assert L.tolcuda_eval_batch_summary(ev.h, 1, x.ctypes.data, ev.n, F.ctypes.data, ev.neF, G.ctypes.data, ev.neG,
                                         S.ctypes.data, 4, flags | T.evaluator.COMPACT_G) == -2     # EUNSUPPORTED
     assert np.isnan(F).all() and np.isnan(G).all()
-    # the release library has no experiment switches: flag bits it does not define are rejected, nothing runs
+    # flag bits the library does not define are rejected, nothing runs
     l0 = ev.launches
     for bad in (0x10000, 0x20000 | flags, 0x800 | flags, 1 << 30):
         assert L.tolcuda_eval_batch(ev.h, 1, x.ctypes.data, ev.n, F.ctypes.data, ev.neF, G.ctypes.data, ev.neG, bad | flags) == -1

@@ -53,34 +53,20 @@ constexpr int MAX_DEVICES = 64;  // power of two; device ordinals are folded int
 constexpr int PX = TOLCUDA_PX;
 constexpr int PF = TOLCUDA_PF;
 constexpr int REC = TOLCUDA_REC;
-// Record buffers.  A drain pass hands NPP windows (lanes NPP*g .. NPP*g+NPP-1) to the TMA unit: each of those
-// lanes places its 33 x-dependent values in its own record slot (the slots' constants are written once per
-// run of trajectories), then lane 0 issues the bulk copies, one per dense run of UNIT records.  The layout is a
-// build-time choice so that variants can be measured side by side (tools/exp/build_variant.sh;
-// profiles/r1_history.md).  Default: one buffer of 8 records per warp, 4 passes per tile, one 6,656-byte
-// bulk copy per pass; a pass waits until the TMA unit has read the previous one.  Against two buffers of 4
-// records (8 passes, fill and read overlapped) this halves the shared-store instructions, proxy fences and
-// warp barriers of a tile for the same shared memory, and measured 0.3 % faster; 16-record buffers would
-// leave room for only one CTA per SM.
-#ifndef TOLCUDA_NPP
-#define TOLCUDA_NPP 8
-#define TOLCUDA_NBUF 1
-#define TOLCUDA_UNIT 8
-#define TOLCUDA_PADW 0
-#endif
-constexpr int NPP = TOLCUDA_NPP;       // windows per drain pass
-constexpr int NBUF = TOLCUDA_NBUF;     // record buffers per warp (2: the TMA unit reads one while lanes fill the other)
-constexpr int UNIT = TOLCUDA_UNIT;     // records per dense run = per bulk copy
-constexpr int PADW = TOLCUDA_PADW;     // doubles between runs (even: runs stay 16-byte aligned)
-constexpr int USTR = UNIT * REC + PADW;                     // run stride
-constexpr int BUF_LEN = (NPP / UNIT) * USTR;
+// Record buffer: one per warp, NPP = 8 dense record slots of REC doubles.  A drain pass hands 8 windows (lanes
+// 8g .. 8g+7) to the TMA unit: each of those lanes places its 33 x-dependent values in its own slot (the slots'
+// constants are written once per run of trajectories), then lane 0 issues the 8 records (6,656 bytes) as one bulk
+// copy; a pass waits until the TMA unit has read the previous one, so a tile takes 4 passes.  Two buffers of 4
+// records (8 passes, fill and read overlapped) need the same shared memory, twice the shared-store instructions,
+// proxy fences and warp barriers of a tile, and measured 0.3 % slower; 16-record buffers leave room for only one
+// CTA per SM and measured slower still (profiles/r1_history.md).
+constexpr int NPP = 8;                 // windows per drain pass = record slots per warp
 // + 16 doubles of slack: when the records of a trajectory start 8 mod 16 in global memory (odd ts, or an odd
 // leading dimension) the slots are used shifted by one double, so that all but the first and the last double of
-// a pass still form one 16-byte aligned bulk copy (see the drain in tile_eval); 16 keeps the tiles 128-byte aligned
+// a pass still form one 16-byte aligned bulk copy (see tile_drain); 16 keeps the tiles 128-byte aligned
 constexpr int TILE_SLACK = 16;
-constexpr int TILE_LEN = NBUF * BUF_LEN + TILE_SLACK;
+constexpr int TILE_LEN = NPP * REC + TILE_SLACK;
 constexpr int SX_LEN = 368;            // a warp's x slice: slot for x[11*k0] + 33 nodes = 364 doubles (tile stays 128-byte aligned)
-static_assert(NPP % UNIT == 0 && 32 % NPP == 0 && PADW % 2 == 0 && NBUF * NPP <= 32, "record buffer layout");
 constexpr int WARP_SMEM = SX_LEN + TILE_LEN;        // kernel A
 constexpr int WARP_SMEM_B = 2 * SX_LEN + TILE_LEN;  // kernel L (and kernel A with runs): two x-slice buffers
 constexpr int F_LD = 10;               // smem stride of a window's 8 defects (== 2 mod 4)
@@ -109,16 +95,6 @@ __host__ __device__ constexpr bool mode_is_op(int mode) { return mode == MODE_JV
 __host__ __device__ constexpr bool mode_has_records(int mode) { return mode == MODE_PLAIN || mode == MODE_SUMMARY; }
 // doubles of a warp's tile in kernel A
 __host__ __device__ constexpr int tile_len_of(int mode) { return mode_is_fonly(mode) ? 0 : TILE_LEN; }
-
-// Kernel experiment switches (bits 2.. of the kernels' needG argument: 4 = stage but do not store G, 8 = no
-// trigonometry, 16 = no Jacobian arithmetic) exist only in the experiments build (make exp -> libtolcuda_exp.so,
-// tools/kbench.py); in the release library they are compiled out and the public flags that would reach them are
-// rejected (tolcuda_api.cpp).
-#ifdef TOLCUDA_EXPERIMENTS
-#define EXP_SWITCH(needG, bit) ((needG) & (bit))
-#else
-#define EXP_SWITCH(needG, bit) 0
-#endif
 
 // Programmatic dependent launch (FgLaunch::pdl).  Every CTA releases the NEXT launch on the stream as soon as it
 // has started (griddepcontrol.launch_dependents), so the next grid's CTAs move into SMs the tail of this grid has
@@ -387,13 +363,13 @@ struct Goal {
 // Record layout (row s of the window at 13*s: [d/d dt, d/d c0..c10 @k, d/d c_s @k+1]).  Structural
 // constants: tabG zero-initialisation and the +-1 entries (src/problem.cpp:1038, 1084, 1098, 1112, 1170,
 // 1182, 1204); everything x-dependent is zeroed here and written per window by record_store.
-// offset of record slot q (0 .. NPP-1) within a record buffer
-__device__ __forceinline__ int slot_offset(const int q) { return (q / UNIT) * USTR + (q % UNIT) * REC; }
-// lanes 0 .. NBUF*NPP-1 each prepare one record slot: zeros, then the 13 structural +-1 entries.
+// offset of record slot q (0 .. NPP-1) within the record buffer
+__device__ __forceinline__ int slot_offset(const int q) { return q * REC; }
+// lanes 0 .. NPP-1 each prepare one record slot: zeros, then the 13 structural +-1 entries.
 // mis = 1: the slots sit one double further (records that start 8 mod 16 in global memory)
 __device__ __forceinline__ void tile_init(double *tile, const int lane, const int mis) {
-    if (lane >= NBUF * NPP) return;
-    double *rec = tile + (lane / NPP) * BUF_LEN + slot_offset(lane % NPP) + mis;
+    if (lane >= NPP) return;
+    double *rec = tile + slot_offset(lane) + mis;
     if (mis) {
         rec[0] = 0.0;
 #pragma unroll
@@ -544,75 +520,60 @@ __device__ __forceinline__ void wind_cube(const FgConst &c, const Num xn, const 
     }
 }
 
-// ---- drain: passes of NPP windows through the record buffer(s), whole records to global (tile_eval) ------------
+// ---- drain: passes of NPP windows through the record buffer, whole records to global (tile_eval) ---------------
 __device__ __forceinline__ void tile_drain(const FgConst &c, double *tile, const uint32_t tile_s, const int k0, const int nk,
-                                           const int lane, double *__restrict__ Gb, const int needG, int &tile_mis,
-                                           const double *v, const double mdt) {
-    // Pass g (windows k0+NPP*g ..) fills buffer g % NBUF once the TMA unit has read what the buffer held
-    // before; lane 0 issues the pass's bulk copies (one per dense run of UNIT records) as one bulk group.
+                                           const int lane, double *__restrict__ Gb, int &tile_mis, const double *v,
+                                           const double mdt) {
+    // Pass g (windows k0+NPP*g ..) fills the buffer once the TMA unit has read the previous pass; lane 0 issues the
+    // pass's records as one bulk copy.
     // Records that start 8 mod 16 in global memory (R0 is odd for odd ts; odd leading dimensions) are staged one
     // double further into the slots: all but the first and the last double of a pass then form one 16-byte
     // aligned bulk copy, and two lanes store those two doubles.
     double *Grec = Gb + c.R0 + (size_t)REC * k0;  // record of window k0
     const int mis = (int)(reinterpret_cast<uintptr_t>(Grec) >> 3) & 1;
-    constexpr bool SHIFTABLE = (UNIT == NPP);  // one dense run per pass (the default layout)
-    const bool bulk = SHIFTABLE || !mis;
-    if (SHIFTABLE && mis != tile_mis) {  // the slots' constants are in place for the other alignment
+    if (mis != tile_mis) {  // the slots' constants are in place for the other alignment
         __syncwarp();
         tile_init(tile, lane, mis);
         tile_mis = mis;
         __syncwarp();
     }
-    const int sh = SHIFTABLE ? mis : 0;
 #pragma unroll 1
     for (int g = 0; g < 32 / NPP; g++) {
         if (g * NPP >= nk) break;
-        double *buf = tile + (g % NBUF) * BUF_LEN;
-        if (bulk && g >= NBUF) {
-            if (lane == 0) bulk_wait_read<NBUF - 1>();  // pass g-NBUF has been read: its buffer is free
+        if (g >= 1) {
+            if (lane == 0) bulk_wait_read<0>();  // pass g-1 has been read: the buffer is free
             __syncwarp();
         }
         if ((lane / NPP) == g) {
-            if (sh) record_store_shifted(buf + slot_offset(lane & (NPP - 1)) + 1, v, mdt);
-            else record_store(buf + slot_offset(lane & (NPP - 1)), v, mdt);
+            if (mis) record_store_shifted(tile + slot_offset(lane & (NPP - 1)) + 1, v, mdt);
+            else record_store(tile + slot_offset(lane & (NPP - 1)), v, mdt);
             // the writers make their generic-proxy stores visible to the async proxy (the TMA unit) ...
-            if (bulk && !EXP_SWITCH(needG, 4)) asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+            asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
         }
         const int nrec = min(NPP, nk - g * NPP);
         double *dst = Grec + (size_t)REC * NPP * g;
-        if (EXP_SWITCH(needG, 4)) {
-            __syncwarp();
-        } else if (bulk) {
-            __syncwarp();  // ... and lane 0 issues the copies after all of them have done so
-            if (sh) {
-                // doubles [1, nrec*REC - 1) of the pass as one aligned copy; lanes 1 and 2 store the two ends
-                if (lane == 0) bulk_store(dst + 1, tile_s + 8 * ((g % NBUF) * BUF_LEN + 2), (nrec * REC - 2) * 8);
-                if (lane == 1) dst[0] = buf[1];
-                if (lane == 2) dst[nrec * REC - 1] = buf[nrec * REC];
-            } else if (lane == 0) {
-#pragma unroll
-                for (int u = 0; u < NPP / UNIT; u++)
-                    if (u * UNIT < nrec)
-                        bulk_issue(dst + u * UNIT * REC, tile_s + 8 * ((g % NBUF) * BUF_LEN + u * USTR), min(UNIT, nrec - u * UNIT) * REC * 8);
-                bulk_commit();
-            }
-        } else {
-            __syncwarp();
-            for (int i = lane; i < nrec * REC; i += 32) dst[i] = buf[(i / (UNIT * REC)) * USTR + i % (UNIT * REC)];
-            __syncwarp();
+        __syncwarp();  // ... and lane 0 issues the copy after all of them have done so
+        if (mis) {
+            // doubles [1, nrec*REC - 1) of the pass as one aligned copy; lanes 1 and 2 store the two ends
+            if (lane == 0) bulk_store(dst + 1, tile_s + 16, (nrec * REC - 2) * 8);
+            if (lane == 1) dst[0] = tile[1];
+            if (lane == 2) dst[nrec * REC - 1] = tile[nrec * REC];
+        } else if (lane == 0) {
+            // nrec is 1 .. NPP here: the guard and the clamp are redundant, but without them ptxas compiles every
+            // record-writing instance differently from the code the profiles were measured on
+            if (0 < nrec) bulk_issue(dst, tile_s, min(NPP, nrec) * REC * 8);
+            bulk_commit();
         }
     }
-    if (bulk) {
-        if (lane == 0) bulk_wait_read<0>();  // the buffers are reused (or released) after this
-        __syncwarp();
-    }
+    if (lane == 0) bulk_wait_read<0>();  // the buffer is reused (or released) after this
+    __syncwarp();
 }
 
 // ---- one warp, one tile of 32 windows ---------------------------------------------------------------
 //
 // sx: the warp's staged x slice (slot 0 = x[11*k0], node j of the slice at sx[1+11j]).  Once every lane
 // has its window in registers the slice is dead and serves as staging area for F and the objective row.
-// tile: the warp's NBUF x NPP record slots, constants already in place (tile_init).
+// tile: the warp's NPP record slots, constants already in place (tile_init).
 // dep_wait: this is the warp's first tile of a launch that may have started before the preceding launch on the
 // stream had finished (pdl_wait before the first global store).
 // MODE_HVP: Db is the trajectory's row of d, Zb its row of z (or null); the window arithmetic runs on Dual, and
@@ -662,13 +623,9 @@ __device__ __forceinline__ void tile_eval(const FgConst &c, double *sx, double *
 
     // ---- shared sub-expressions of the window ----
     Num sc, cc, sg, cg, sp, cp;
-    if (EXP_SWITCH(needG, 8)) {
-        sc = sg = sp = 0.6, cc = cg = cp = 0.8;
-    } else {
-        sincos(chi, &sc, &cc);
-        sincos(gam, &sg, &cg);
-        sincos(phi, &sp, &cp);
-    }
+    sincos(chi, &sc, &cc);
+    sincos(gam, &sg, &cg);
+    sincos(phi, &sp, &cp);
     // wind, NED <- ENU (src/problem.cpp:970-981): Wx = v, dWx_dx = dv_dy, dWx_dy = dv_dx, dWx_dz = -dv_dz;
     // every other component is exactly zero under models 0, 1 and 3.
     //   model 1 (:522-524): v = -Vref*zs/href with zs = -z, dv_dz = -Vref/href
@@ -831,10 +788,6 @@ __device__ __forceinline__ void tile_eval(const FgConst &c, double *sx, double *
 
     // ---- Jacobian rows, src/problem.cpp:1074-1192 ----
     Num v[NVAR];
-    if (EXP_SWITCH(needG, 16)) {  // experiment switch: no Jacobian arithmetic, the drain alone
-#pragma unroll
-        for (int i = 0; i < NVAR; i++) v[i] = Va + (double)i;
-    } else {
     v[0] = -vx;  // F1 :1084-1088
     v[1] = mdt * cc * cg;
     v[2] = Vadt * cc * sg;
@@ -892,15 +845,12 @@ __device__ __forceinline__ void tile_eval(const FgConst &c, double *sx, double *
     }
     v[29] = -dphi;  // F7 :1172
     v[30] = -dCL;   // F8 :1184
-    }
-#ifndef TOLCUDA_OP_NOPIN
     if constexpr (OP && MODE != MODE_HVP) {
         // the 31 entries meet in registers before the products consume them: left free, ptxas interleaves their
         // arithmetic with the dot products and spills at the 128-register cap
 #pragma unroll
         for (int i = 0; i < NVAR; i++) asm volatile("" : "+d"(v[i]));
     }
-#endif
 
     if constexpr (MODE == MODE_JVP) {
         // y = J d for this warp's rows: the window's 8 defect rows (src/problem.cpp:1074-1192 entries times the
@@ -1035,7 +985,7 @@ __device__ __forceinline__ void tile_eval(const FgConst &c, double *sx, double *
         return;
     }
 
-    if constexpr (mode_has_records(MODE)) tile_drain(c, tile, tile_s, k0, nk, lane, Gb, needG, tile_mis, v, mdt);
+    if constexpr (mode_has_records(MODE)) tile_drain(c, tile, tile_s, k0, nk, lane, Gb, tile_mis, v, mdt);
 }
 
 // ---- end of a trajectory: F[0], boundary rows, objective-row ends --------------------------------------
@@ -1274,10 +1224,7 @@ constexpr int MAXPER = 4;
 // (1,000 W; profiles/r4_opbench_hvp.txt): 4 (128 registers, 130-1,030 bytes of spill) 1.91 ms on S10 ts=200 at
 // B=65,536 and 80 us on G7 ts=100 at B=4,096; 3 (168 / 255 registers) 2.34 ms / 90.5 us; 2 (255 registers, no
 // spill but 8 warps per SM) 2.34 ms / 109 us: the dual arithmetic wants warps more than registers
-#ifndef TOLCUDA_HVP_MINB
-#define TOLCUDA_HVP_MINB 4
-#endif
-constexpr int HVP_MINB = TOLCUDA_HVP_MINB;
+constexpr int HVP_MINB = 4;
 template <int FORM, int WIND, int MAXT, int MINB, int MODE, bool LOOP, bool GOALS>
 __device__ __forceinline__ void fg_cta_body(const FgConst &c, int nrun, int per_arg, const double *__restrict__ x, long ldx,
                                             double *__restrict__ F, long ldF, double *__restrict__ G, long ldG, int needF,
@@ -1312,14 +1259,8 @@ __device__ __forceinline__ void fg_cta_body(const FgConst &c, int nrun, int per_
     const bool run = LOOP && bid < nrun;
     const size_t b0 = LOOP ? (run ? (size_t)per * bid : (size_t)per * nrun + (size_t)(bid - nrun)) : (size_t)bid;
     const int ntraj = run ? per : 1;
-#ifdef TOLCUDA_BALANCE  // experiment: the same number of windows for every warp instead of full tiles and a remainder
-    const int tw = (ts + nwarps - 1) / nwarps;
-    const int k0 = tw * warp;
-    const int nk = min(tw, ts - k0);
-#else
     const int k0 = 32 * warp;
     const int nk = min(32, ts - k0);
-#endif
     const int cnt = 1 + PX * (nk + 1);           // doubles of a slice
     const double *xw = x + b0 * ldx + (size_t)PX * k0;  // this warp's slice of the run's first trajectory
     slice_prefetch(wsm_s, xw, cnt, lane);
@@ -1335,7 +1276,7 @@ __device__ __forceinline__ void fg_cta_body(const FgConst &c, int nrun, int per_
     // later trajectory's differs: odd leading dimension)
     int tile_mis = 0;
     if (mode_has_records(MODE)) {
-        if (UNIT == NPP) tile_mis = (int)(reinterpret_cast<uintptr_t>(G + b0 * ldG + c.R0 + (size_t)REC * k0) >> 3) & 1;
+        tile_mis = (int)(reinterpret_cast<uintptr_t>(G + b0 * ldG + c.R0 + (size_t)REC * k0) >> 3) & 1;
         if (needG) tile_init(tile, lane, tile_mis);
     }
     if (tid < MAXPER) arrivals[tid] = 0;
@@ -1491,7 +1432,7 @@ __device__ __forceinline__ void fg_long_body(const FgConst &c, const double *__r
     }
     int tile_mis = 0;
     if (mode_has_records(MODE)) {
-        if (UNIT == NPP) tile_mis = (int)(reinterpret_cast<uintptr_t>(Gb + c.R0) >> 3) & 1;  // REC*k0 is even
+        tile_mis = (int)(reinterpret_cast<uintptr_t>(Gb + c.R0) >> 3) & 1;  // REC*k0 is even
         if (needG) tile_init(tile, lane, tile_mis);
     }
     if (tid == 0) arrivals = 0;
@@ -1566,10 +1507,7 @@ fg_long_kernel(const __grid_constant__ FgConst c, const double *__restrict__ x, 
 }
 
 // MODE_HVP, as fg_cta_hvp_kernel
-#ifndef TOLCUDA_HVP_LMINB
-#define TOLCUDA_HVP_LMINB 1
-#endif
-constexpr int HVP_LMINB = TOLCUDA_HVP_LMINB;
+constexpr int HVP_LMINB = 1;
 template <int FORM, int WIND>
 __global__ void __launch_bounds__(LWARPS * 32, HVP_LMINB)
 fg_long_hvp_kernel(const __grid_constant__ FgConst c, const double *__restrict__ x, long ldx, double *__restrict__ lam,
@@ -1599,23 +1537,30 @@ cudaError_t launch_kernel(Kern kern, const int grid, const int nthr, const size_
     return cudaLaunchKernelEx(&cfg, kern, args...);
 }
 
+// lets KERN use smem bytes of dynamic shared memory on the launch's device.  The attribute is per device, so the cache of
+// what has been set is too (tolbatch drives one device per thread), and one per kernel instance (KERN).
+template <auto KERN>
+cudaError_t reserve_smem(const FgLaunch &L, const size_t smem) {
+    static std::atomic<size_t> configured[MAX_DEVICES];
+    std::atomic<size_t> &done = configured[L.device & (MAX_DEVICES - 1)];
+    if (smem > done.load(std::memory_order_acquire)) {
+        cudaError_t e = cudaFuncSetAttribute(KERN, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        if (e != cudaSuccess) return e;
+        done.store(smem, std::memory_order_release);
+    }
+    return cudaSuccess;
+}
+
 template <int FORM, int WIND, int MAXT, int MINB, int MODE, bool LOOP, bool GOALS>
 cudaError_t launch_cta_as(const FgLaunch &L, const int per, const int nsingle) {
-    auto kern = [] {
+    constexpr auto kern = [] {
         if constexpr (MODE == MODE_HVP) return fg_cta_hvp_kernel<FORM, WIND, MAXT, MINB, LOOP>;
         else if constexpr (GOALS) return fg_cta_goals_kernel<FORM, WIND, MAXT, MINB, MODE, LOOP>;
         else return fg_cta_kernel<FORM, WIND, MAXT, MINB, MODE, LOOP>;
     }();
     const int nthr = 32 * ((L.c->ts + 31) / 32);
     const size_t smem = sizeof(double) * (size_t)(nthr / 32) * ((per > 1 ? 2 : 1) * SX_LEN + tile_len_of(MODE));
-    // the attribute is per device (and this static per instantiation): tolbatch drives one device per thread
-    static std::atomic<size_t> configured[MAX_DEVICES];
-    std::atomic<size_t> &done = configured[L.device & (MAX_DEVICES - 1)];
-    if (smem > done.load(std::memory_order_acquire)) {
-        cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        if (e != cudaSuccess) return e;
-        done.store(smem, std::memory_order_release);
-    }
+    if (cudaError_t e = reserve_smem<kern>(L, smem)) return e;
     const int nrun = LOOP ? (L.B - nsingle) / per : 0;  // nsingle makes this exact (launch_cta)
     const int grid = LOOP ? nrun + nsingle : L.B;
     if constexpr (MODE == MODE_HVP)
@@ -1647,7 +1592,7 @@ cudaError_t launch_cta(const FgLaunch &L) {
 
 template <int FORM, int WIND, int MODE, bool GOALS>
 cudaError_t launch_long(const FgLaunch &L) {
-    auto kern = [] {
+    constexpr auto kern = [] {
         if constexpr (MODE == MODE_HVP) return fg_long_hvp_kernel<FORM, WIND>;
         else if constexpr (GOALS) return fg_long_goals_kernel<FORM, WIND, MODE>;
         else return fg_long_kernel<FORM, WIND, MODE>;
@@ -1658,13 +1603,7 @@ cudaError_t launch_long(const FgLaunch &L) {
     int nthr = 32 * ((nt + rounds - 1) / rounds);
     if (L.lwarps > 0) nthr = 32 * (L.lwarps < nt ? L.lwarps : nt);  // tolcuda_set_option "lwarps"
     const size_t smem = sizeof(double) * (size_t)(nthr / 32) * WARP_SMEM_B;
-    static std::atomic<size_t> configured[MAX_DEVICES];  // per device, see launch_cta_as
-    std::atomic<size_t> &done = configured[L.device & (MAX_DEVICES - 1)];
-    if (smem > done.load(std::memory_order_acquire)) {
-        cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        if (e != cudaSuccess) return e;
-        done.store(smem, std::memory_order_release);
-    }
+    if (cudaError_t e = reserve_smem<kern>(L, smem)) return e;
     if constexpr (MODE == MODE_HVP)
         return launch_kernel(kern, L.B, nthr, smem, L, *L.c, L.x, L.ldx, L.F, L.ldF, L.G, L.ldG, L.D, L.ldD, L.Z, L.ldZ);
     else if constexpr (GOALS)
@@ -1702,10 +1641,8 @@ cudaError_t launch_sel(const FgLaunch &L) {
 template <int FORM, int WIND, bool GOALS>
 cudaError_t launch_flavour(const FgLaunch &L) {
     if (L.compact) return launch_sel<FORM, WIND, MODE_COMPACT, GOALS>(L);
-#ifndef TOLCUDA_NO_FONLY  // (variant builds measure the plain flavour on F-only calls)
     if (!L.needG && L.kernel != 2 && L.c->ts <= 256)
         return L.S ? launch_sel<FORM, WIND, MODE_FSUMM, GOALS>(L) : launch_sel<FORM, WIND, MODE_FONLY, GOALS>(L);
-#endif
     return L.S ? launch_sel<FORM, WIND, MODE_SUMMARY, GOALS>(L) : launch_sel<FORM, WIND, MODE_PLAIN, GOALS>(L);
 }
 

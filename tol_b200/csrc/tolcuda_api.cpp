@@ -4,7 +4,6 @@
 #include <cuda_runtime.h>
 
 #include <algorithm>
-#include <cctype>
 #include <atomic>
 #include <cstdint>
 #include <cstdio>
@@ -63,9 +62,7 @@ struct tolcuda_ctx {
     tolcuda_config cfg;
     FgConst c;
     int kernel = 0;
-    // launch shape (fg_kernels.cu launch_sel / launch_cta), see tolcuda_set_option.  The experiments build (make exp)
-    // also reads them from the environment: TOLCUDA_KERNEL, TOLCUDA_PER, TOLCUDA_PER_MIN_WAVES, TOLCUDA_TAIL_X4,
-    // TOLCUDA_LWARPS, TOLCUDA_ZEROCOPY, TOLCUDA_COMPACT, TOLCUDA_CHUNK_MB
+    // launch shape (fg_kernels.cu launch_sel / launch_cta), set through tolcuda_set_option only
     int per = 2;             // trajectories per CTA for large batches
     int per_auto = 1;        // ... and one per CTA below per_min_waves waves of CTAs
     int per_min_waves = -1;  // -1: 24 (8 for launches that overlap their predecessor: tools/sweep.py, profiles/r2_sweep.txt)
@@ -379,15 +376,6 @@ int tolcuda_create(const tolcuda_config *cfg, tolcuda_handle *out) {
     }
     pattern_build(c.form, c.ts, h->iG, h->jG);
 
-#ifdef TOLCUDA_EXPERIMENTS
-    for (const char *name : {"kernel", "per", "per_min_waves", "tail_x4", "lwarps", "zero_copy", "compact_host", "chunk_mb", "full_rows_pct"}) {
-        std::string env = std::string("TOLCUDA_") + name;
-        for (char &ch : env) ch = (char)std::toupper((unsigned char)ch);
-        if (env == "TOLCUDA_ZERO_COPY") env = "TOLCUDA_ZEROCOPY";
-        if (env == "TOLCUDA_COMPACT_HOST") env = "TOLCUDA_COMPACT";
-        if (const char *v = std::getenv(env.c_str())) tolcuda_set_option(h, name, std::atol(v));
-    }
-#endif
     if (const char *env = std::getenv("TOLCUDA_DUMP_DIR")) h->dump_dir = env;
 
     int rc = 0;
@@ -653,16 +641,11 @@ static int eval_batch(tolcuda_handle h, int B, const double *x, long ldx, double
                       double *summary, long lds, int flags, const double *goals) {
     if (!h || B < 0 || (summary && lds < 4)) return TOLCUDA_EINVAL;
     const int needF = (flags & TOLCUDA_NEED_F) != 0;
-#ifdef TOLCUDA_EXPERIMENTS
-    // experiments build only: bits 16.. of flags are kernel experiment switches (tools/kbench.py)
-    const int needG = (flags & TOLCUDA_NEED_G) ? (1 | (((flags >> 16) & 0xff) << 1)) : 0;
-#else
     if (flags & ~TOLCUDA_FLAGS_ALL) {
         set_error("tolcuda_eval_batch: unknown flag bits");
         return TOLCUDA_EINVAL;
     }
     const int needG = (flags & TOLCUDA_NEED_G) != 0;
-#endif
     if (B == 0 || (!needF && !needG && !summary)) return 0;
     const FgConst &c = h->c;
     const long lenGc = compact_len(c.form, c.ts);

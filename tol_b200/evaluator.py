@@ -306,15 +306,14 @@ class Evaluator:
                                            F.strides[0] // 8, G.ctypes.data, G.strides[0] // 8, flags))
         return F, G
 
-    def eval_batch_device(self, X, F, G, needF=True, needG=True, sync=True, compact_rows=False, overlap=0, extra_flags=0):
+    def eval_batch_device(self, X, F, G, needF=True, needG=True, sync=True, compact_rows=False, overlap=0):
         """tolcuda_eval_batch with torch CUDA tensors [B, ld] (float64, row-contiguous).  overlap (sync=False only):
-        1 = TOLCUDA_OVERLAP, 2 = TOLCUDA_OVERLAP_DISJOINT.  extra_flags: ORed in as is (tools/kbench.py with the
-        experiments build; the release library rejects unknown bits)"""
+        1 = TOLCUDA_OVERLAP, 2 = TOLCUDA_OVERLAP_DISJOINT"""
         self._follow_torch(X)
         B = X.shape[0]
         flags = (NEED_F if needF else 0) | (NEED_G if needG else 0) | DEVICE_PTRS | (0 if sync else NO_SYNC)
         flags |= COMPACT_G if compact_rows else 0
-        flags |= (OVERLAP if overlap == 1 else 0) | (OVERLAP_DISJOINT if overlap == 2 else 0) | int(extra_flags)
+        flags |= (OVERLAP if overlap == 1 else 0) | (OVERLAP_DISJOINT if overlap == 2 else 0)
         _l.check(self.L.tolcuda_eval_batch(self.h, B, X.data_ptr(), X.stride(0), F.data_ptr(), F.stride(0),
                                            G.data_ptr(), G.stride(0), flags))
 

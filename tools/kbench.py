@@ -1,10 +1,8 @@
 #!/usr/bin/env python
 """Kernel-only timing helper (device-resident, CUDA events on the launching stream): used to compare
 kernel variants and as the short command that is run under ncu.  Not the bench contract -- bench.py is.
-The work-skipping switches (--need FG4 / FG8 / FG16) exist only in the experiments build: `make -C tol_b200/csrc exp`
-and run with TOLCUDA_LIB=tol_b200/libtolcuda_exp.so; the release library rejects them.
 
-    python tools/kbench.py --workload S10_tempest_ts200 --batch 16384 --steps 10 [--npp 8]"""
+    python tools/kbench.py --workload S10_tempest_ts200 --batch 16384 --steps 10"""
 import argparse
 import json
 import os
@@ -26,7 +24,7 @@ ap.add_argument("--per", type=int, default=0)
 ap.add_argument("--tail-x4", type=int, default=-1)
 ap.add_argument("--overlap", type=int, default=0, help="1: TOLCUDA_OVERLAP, 2: TOLCUDA_OVERLAP_DISJOINT (two result buffer sets)")
 ap.add_argument("--goff", type=int, default=0, help="shift the G buffer by this many doubles (alignment experiments)")
-ap.add_argument("--need", default="FG")
+ap.add_argument("--need", default="FG", help="F, FG, or S (the per-trajectory summary alone)")
 ap.add_argument("--distinct", type=int, default=512, help="distinct synthetic trajectories (tiled)")
 ap.add_argument("--ts", type=int, default=0, help="override the number of windows (x0 = the restated InitialCond for that ts)")
 args = ap.parse_args()
@@ -60,18 +58,14 @@ Gs = [torch.empty(B * ldG + 64, dtype=torch.float64, device="cuda")[args.goff:ar
 st = torch.cuda.Stream()
 ev.set_stream(st.cuda_stream)
 needF, needG = "F" in args.need, "G" in args.need
-extra = 0
-if needG:  # experiment switches (experiments build only): FG4 = no G stores, FG8 = no trig, FG16 = no Jacobian arithmetic, sums allowed (FG24)
-    digits = "".join(ch for ch in args.need if ch.isdigit())
-    extra = ((int(digits) if digits else 0) >> 1) << 16
 with torch.cuda.stream(st):
     for i in range(args.warmup):
-        ev.eval_batch_device(Xd, Fs[i % nset], Gs[i % nset], needF, needG, sync=False, overlap=args.overlap, extra_flags=extra)
+        ev.eval_batch_device(Xd, Fs[i % nset], Gs[i % nset], needF, needG, sync=False, overlap=args.overlap)
     torch.cuda.synchronize()
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record(st)
     for i in range(args.steps):
-        ev.eval_batch_device(Xd, Fs[i % nset], Gs[i % nset], needF, needG, sync=False, overlap=args.overlap, extra_flags=extra)
+        ev.eval_batch_device(Xd, Fs[i % nset], Gs[i % nset], needF, needG, sync=False, overlap=args.overlap)
     e1.record(st)
     torch.cuda.synchronize()
 ms = e0.elapsed_time(e1) / args.steps
