@@ -254,8 +254,8 @@ int tolcuda_jac_tvec(tolcuda_handle h, int B, const double *x, long ldx, const d
  * consume them in registers, moving 8*(3n + neF) bytes per trajectory (+ 8n with z).
  * Device pointers on the context's device; flags: 0 or TOLCUDA_NO_SYNC (TOLCUDA_HOST_PTRS: TOLCUDA_EUNSUPPORTED).  A
  * null x, lambda, d or w, or a leading dimension shorter than its row, is TOLCUDA_EINVAL; B = 0 launches nothing.
- * Evaluated with the context's goal; the options "kernel", "per", "lwarps" and "per_min_waves" apply as to
- * tolcuda_jac_tvec, and every option gives the same bits except w[0] and z[0] (sums over the trajectory) under
+ * Evaluated with the context's goal (tolcuda_lag_hess_vec_goals: one per trajectory); the options "kernel", "per",
+ * "lwarps" and "per_min_waves" apply as to tolcuda_jac_tvec, and every option gives the same bits except w[0] and z[0] (sums over the trajectory) under
  * kernel L. */
 int tolcuda_lag_hess_vec(tolcuda_handle h, int B, const double *x, long ldx, const double *lambda, long ldl,
                          const double *d, long ldd, double *w, long ldw, double *z, long ldz, int flags);
@@ -308,16 +308,27 @@ int tolcuda_eval_batch_summary(tolcuda_handle h, int B, const double *x, long ld
  *   tolcuda_set_goals         keeps a goal table on the context's device: row b is goal[b*ldg + 0..3] = xg, yg, zg, rg
  *                             in NED, as tolcuda_config.goal (ldg >= 4; host memory).  chi_d is derived per row on the
  *                             host exactly as tolcuda_create derives it.  Synchronises the context's stream before it
- *                             replaces the previous table, so TOLCUDA_NO_SYNC launches in flight finish with the table
- *                             they were enqueued with.  count = 0 frees the table.
+ *                             replaces the previous table, so TOLCUDA_NO_SYNC launches in flight (evaluations and
+ *                             products) finish with the table they were enqueued with.  count = 0 frees the table.
  *   tolcuda_eval_batch_goals  as tolcuda_eval_batch_summary (summary may be NULL; every flag and option of it applies),
  *                             but trajectory b of this call uses goal row row0 + b of the table.
- * Row b of F, G and summary is bit for bit what a context created with row0 + b's goal (and the same options) writes
- * for the same x.  No table, row0 < 0 or row0 + B > count (and a NULL handle) return TOLCUDA_EINVAL and launch nothing.
- * The table lives in device memory: 64 bytes per row. */
+ *   tolcuda_jac_vec_goals, tolcuda_jac_tvec_goals, tolcuda_lag_hess_vec_goals
+ *                             as tolcuda_jac_vec, tolcuda_jac_tvec and tolcuda_lag_hess_vec (same arguments after B, same
+ *                             validation, flags and options; one launch per call), but trajectory b of this call uses
+ *                             goal row row0 + b of the table: the matrix-free products of a batch of different missions.
+ * Row b of F, G and summary (of y, z, w and the optional z) is bit for bit what a context created with row0 + b's goal
+ * (and the same options) writes for the same x (and d, lambda); under kernel L the caveat of tolcuda_lag_hess_vec on
+ * w[0] and z[0] applies unchanged.  No table, row0 < 0 or row0 + B > count (and a NULL handle, checked before any
+ * CUDA call) return TOLCUDA_EINVAL and launch nothing.  The table lives in device memory: 64 bytes per row. */
 int tolcuda_set_goals(tolcuda_handle h, long count, const double *goal, long ldg);
 int tolcuda_eval_batch_goals(tolcuda_handle h, long row0, int B, const double *x, long ldx, double *F, long ldF,
                              double *G, long ldG, double *summary, long lds, int flags);
+int tolcuda_jac_vec_goals(tolcuda_handle h, long row0, int B, const double *x, long ldx, const double *d, long ldd,
+                          double *y, long ldy, int flags);
+int tolcuda_jac_tvec_goals(tolcuda_handle h, long row0, int B, const double *x, long ldx, const double *lambda, long ldl,
+                           double *z, long ldz, int flags);
+int tolcuda_lag_hess_vec_goals(tolcuda_handle h, long row0, int B, const double *x, long ldx, const double *lambda,
+                               long ldl, const double *d, long ldd, double *w, long ldw, double *z, long ldz, int flags);
 
 /* page-locked host memory for x/F/G of the host-pointer batch path (full PCIe speed, asynchronous
  * copies); plain wrappers so that a C/C++ driver needs no CUDA headers */

@@ -330,6 +330,10 @@ __device__ __forceinline__ void bulk_wait_read() {
 // stay readable through the trajectory's epilogue.  They are read from there at each use, not held in registers.
 // Kernel L stages them for S10 only, whose tiles read them; G7 reads them once per trajectory, in the epilogue, from
 // the table row itself (a pointer to the staged values, live across the tile loop, spills in the wind-cube instances).
+// The operator modes (MODE_JVP, MODE_VJP, MODE_HVP) have no instances for a goal table: they always read their goal
+// from a row, goals + gld*b (a goal table's rows, or the context's own goal row with gld = 0), and read it from the row
+// itself (ROW) in both kernels.  Staged beside the slice in kernel A, it cost registers in the run-loop instances:
+// the J d ones of wind model 1 started to spill (4-8 bytes), where reading the row does not.
 constexpr int GOAL_SX = SX_LEN - 4;
 static_assert(1 + PX * 33 <= GOAL_SX && 32 * F_LD <= GOAL_SX && 3 * 33 <= GOAL_SX, "goal values overlap the slice");
 template <int FORM>
@@ -578,13 +582,15 @@ __device__ __forceinline__ void tile_drain(const FgConst &c, double *tile, const
 // stream had finished (pdl_wait before the first global store).
 // MODE_HVP: Db is the trajectory's row of d, Zb its row of z (or null); the window arithmetic runs on Dual, and
 // ts_out.sumT / ts_out.sump return the tile's shares of z[0] / w[0].
-template <int FORM, int WIND, int MODE, bool GOALS>
+// ROW: the goal is read from the table row grow (the operator modes), not from beside the slice
+template <int FORM, int WIND, int MODE, bool GOALS, bool ROW = false>
 __device__ __forceinline__ void tile_eval(const FgConst &c, double *sx, double *tile, const uint32_t tile_s, const double dt_in,
                                           const int k0, const int nk, const int lane,
                                           double *__restrict__ Fb, double *__restrict__ Gb,
                                           const int needF, const int needG, TileSums &ts_out,
                                           const bool dep_wait, int &tile_mis, const double *aux = nullptr,
-                                          const double *__restrict__ Db = nullptr, double *__restrict__ Zb = nullptr) {
+                                          const double *__restrict__ Db = nullptr, double *__restrict__ Zb = nullptr,
+                                          const double *grow = nullptr) {
     double &sumT = ts_out.sumT, &sump = ts_out.sump;
     constexpr bool OP = mode_is_op(MODE);
     using Num = std::conditional_t<MODE == MODE_HVP, Dual, double>;
@@ -606,7 +612,7 @@ __device__ __forceinline__ void tile_eval(const FgConst &c, double *sx, double *
     constexpr bool X3 = (WIND == 3);             // wind cube: Wx with all three gradient components
     constexpr bool W = (WIND == 1) || X3;        // Wx and dWx/dz present
     constexpr bool S10 = (FORM == TOLCUDA_FORM_S10);
-    const Goal<FORM, GOALS> gl{sx + GOAL_SX};
+    const Goal<FORM, GOALS, ROW> gl{ROW ? grow : sx + GOAL_SX};
     const int ts = c.ts;
     const int k = k0 + lane;
     const bool active = lane < nk;
@@ -1132,21 +1138,24 @@ __device__ __forceinline__ EndNodes<Num> end_nodes(const FgConst &c, const int l
 // multipliers add to z at node 0 (aux[0..10]) and node ts (aux[11..21]); executed by the tile's whole warp, aux is
 // the warp's own (otherwise unused) record buffer.  Num = Dual (MODE_HVP): the same terms and their derivatives
 // along d, as 22 Duals
-template <int FORM, class Num = double>
-__device__ __forceinline__ void op_aux(const FgConst &c, const int lane, const double dt_in, const double n0_in,
+template <int FORM, class Num, class GoalT>
+__device__ __forceinline__ void op_aux(const FgConst &c, const GoalT gl, const int lane, const double dt_in, const double n0_in,
                                        const double ne_in, const double *__restrict__ lamrow, double *aux_out,
                                        const double *__restrict__ Db = nullptr) {
+    // G7's goal values first: read from the goal row, their latency overlaps that of lambda's loads (constants of
+    // the dual arithmetic)
+    double cd = 0.0, sd = 0.0;
+    if constexpr (FORM == TOLCUDA_FORM_G7) cd = gl.cos_chid(c), sd = gl.sin_chid(c);
     const EndNodes<Num> en = end_nodes<Num>(c, lane, dt_in, n0_in, ne_in, Db);
     const Num dt = en.dt, n0 = en.n0, ne = en.ne;
     Num *aux = reinterpret_cast<Num *>(aux_out);
     const double lb = lane < c.nb ? __ldg(lamrow + (c.neF - c.nb) + lane) : 0.0;
     Num a0 = -lb, a1 = lb;  // rows [dt: 0, (0,c): -1, (ts,c): +1], src/problemS10.cpp:395-415, src/problemG7.cpp:404-511
-    if (FORM == TOLCUDA_FORM_G7) {
+    if constexpr (FORM == TOLCUDA_FORM_G7) {
         const double lam0 = __ldg(lamrow);
         const G7Ends<Num> e = g7_ends(c, dt, n0, ne);
         const double lb0 = __shfl_sync(0xffffffffu, lb, 0), lb1 = __shfl_sync(0xffffffffu, lb, 1);
         const double lb11 = __shfl_sync(0xffffffffu, lb, 11);
-        const double cd = c.cos_chid, sd = c.sin_chid;
         if (lane == 0) {
             a0 = lam0 * e.gx0 + lb0 * (-1.0 + e.ex * cd) + lb1 * (e.ex * sd) + lb11 * (-e.ex);
             a1 = lam0 * (-e.gx0) + lb0 * (1.0 - e.ex * cd) + lb1 * (-(e.ex * sd)) + lb11 * e.ex;
@@ -1160,9 +1169,9 @@ __device__ __forceinline__ void op_aux(const FgConst &c, const int lane, const d
 
 // end of a trajectory in the operator modes, one whole warp; tot: the trajectory's sum of the tiles' shares
 // (MODE_JVP: objective-row entries times d; MODE_VJP, MODE_HVP: the d/d dt column times lambda; MODE_HVP: totd, the
-// derivative of that sum)
-template <int FORM, int MODE>
-__device__ __forceinline__ void op_epilogue(const FgConst &c, const int lane, const double dt, const double tot,
+// derivative of that sum); gl: the trajectory's goal
+template <int FORM, int MODE, class GoalT>
+__device__ __forceinline__ void op_epilogue(const FgConst &c, const GoalT gl, const int lane, const double dt, const double tot,
                                             const double n0, const double ne, double *__restrict__ Fb,
                                             double *__restrict__ Gb, const double totd = 0.0,
                                             const double *__restrict__ Db = nullptr, double *__restrict__ Zb = nullptr) {
@@ -1173,14 +1182,14 @@ __device__ __forceinline__ void op_epilogue(const FgConst &c, const int lane, co
         double d0 = 0.0, de = 0.0;
         if (lane < PX) d0 = __ldg(Gb + 1 + lane), de = __ldg(Gb + 1 + (size_t)PX * ts + lane);
         double *ybnd = Fb + (c.neF - c.nb);
-        if (S10) {
+        if constexpr (S10) {
             if (lane == 0) Fb[0] = c.kdt * ddt + tot;
             if (lane < PX) ybnd[lane] = de - d0;
         } else {
             const G7Ends<double> e = g7_ends(c, dt, n0, ne);
             const double d0x = __shfl_sync(0xffffffffu, d0, 0), d0y = __shfl_sync(0xffffffffu, d0, 1);
             const double dex = __shfl_sync(0xffffffffu, de, 0), dey = __shfl_sync(0xffffffffu, de, 1);
-            const double cd = c.cos_chid, sd = c.sin_chid;
+            const double cd = gl.cos_chid(c), sd = gl.sin_chid(c);
             if (lane == 0) {
                 Fb[0] = (c.kp_ts / e.dist) * ddt + e.gx0 * d0x + e.gy0 * d0y + tot + (-e.gx0) * dex + (-e.gy0) * dey;
                 ybnd[0] = (-1.0 + e.ex * cd) * d0x + (e.ey * cd) * d0y + (1.0 - e.ex * cd) * dex + (-(e.ey * cd)) * dey;
@@ -1218,7 +1227,9 @@ __device__ __forceinline__ void op_epilogue(const FgConst &c, const int lane, co
 // (S10 ts=200, B=65,536): per = 1 2.174 ms, 2 2.068, 3 2.098, 4 2.113, 6 2.156, 8 2.185 (longer runs leave a
 // longer tail at the end of the grid); per = 2 is the default (tolcuda_set_option "per").
 // The body is shared by the instances with the context's goal (fg_cta_kernel) and those with a goal table
-// (fg_cta_goals_kernel, GOALS: goals = row 0 of the launch's rows of the table).
+// (fg_cta_goals_kernel, GOALS: goals = row 0 of the launch's rows of the table).  The operator modes always run with
+// GOALS and read trajectory b's goal from the row goals + gld*b (gld = TOLCUDA_GOAL_LD for a goal table, 0 for the
+// context's own goal row), so a goal table needs no instances of them.
 constexpr int MAXPER = 4;
 // MODE_HVP instances of kernel A: CTAs of 128 threads per SM (256 threads: half as many).  Measured on one B200
 // (1,000 W; profiles/r4_opbench_hvp.txt): 4 (128 registers, 130-1,030 bytes of spill) 1.91 ms on S10 ts=200 at
@@ -1229,8 +1240,9 @@ template <int FORM, int WIND, int MAXT, int MINB, int MODE, bool LOOP, bool GOAL
 __device__ __forceinline__ void fg_cta_body(const FgConst &c, int nrun, int per_arg, const double *__restrict__ x, long ldx,
                                             double *__restrict__ F, long ldF, double *__restrict__ G, long ldG, int needF,
                                             int needG, int flow, double *__restrict__ S, long ldS,
-                                            const double *__restrict__ goals, const double *__restrict__ dm = nullptr,
-                                            long ldd = 0, double *__restrict__ zm = nullptr, long ldz = 0) {
+                                            const double *__restrict__ goals, long gld,
+                                            const double *__restrict__ dm = nullptr, long ldd = 0,
+                                            double *__restrict__ zm = nullptr, long ldz = 0) {
     pdl_release();
     constexpr bool SUMM = mode_has_summary(MODE);
     extern __shared__ __align__(16) double smem[];
@@ -1264,7 +1276,7 @@ __device__ __forceinline__ void fg_cta_body(const FgConst &c, int nrun, int per_
     const int cnt = 1 + PX * (nk + 1);           // doubles of a slice
     const double *xw = x + b0 * ldx + (size_t)PX * k0;  // this warp's slice of the run's first trajectory
     slice_prefetch(wsm_s, xw, cnt, lane);
-    if (GOALS) goal_prefetch<FORM>(wsm_s, goals + TOLCUDA_GOAL_LD * b0, lane);
+    if (GOALS && !OP) goal_prefetch<FORM>(wsm_s, goals + gld * b0, lane);
     cp_async_commit();
     // dt, node 0 and node ts of a trajectory are requested one trajectory ahead, like its slice
     double dt_nx = __ldg(xw - (size_t)PX * k0), n0_nx = 0.0, ne_nx = 0.0;
@@ -1290,10 +1302,10 @@ __device__ __forceinline__ void fg_cta_body(const FgConst &c, int nrun, int per_
         if (t + 1 < ntraj) {
             const double *xn = xw + (t + 1) * ldx;
             slice_prefetch(wsm_s + 8 * (slot ^ 1) * SX_LEN, xn, cnt, lane);
-            if (GOALS) {
+            if (GOALS && !OP) {
                 // G7: the epilogue of trajectory t-1 (lane 0 alone, without G) has read its goal values in that buffer
                 if (FORM != TOLCUDA_FORM_S10) __syncwarp();
-                goal_prefetch<FORM>(wsm_s + 8 * (slot ^ 1) * SX_LEN, goals + TOLCUDA_GOAL_LD * (b + 1), lane);
+                goal_prefetch<FORM>(wsm_s + 8 * (slot ^ 1) * SX_LEN, goals + gld * (b + 1), lane);
             }
             dt_nx = __ldg(xn - (size_t)PX * k0);
             if (lane < PX) {
@@ -1309,11 +1321,13 @@ __device__ __forceinline__ void fg_cta_body(const FgConst &c, int nrun, int per_
         double *Zb = HVP && zm ? zm + b * ldz : nullptr;
         TileSums tsum;
         if ((MODE == MODE_VJP || HVP) && (k0 == 0 || k0 + nk == ts)) {  // the warps that own node 0 / node ts (warp-uniform)
-            op_aux<FORM, std::conditional_t<HVP, Dual, double>>(c, lane, dt, n0, ne, Fb, tile, Db);
+            op_aux<FORM, std::conditional_t<HVP, Dual, double>>(c, Goal<FORM, GOALS, true>{goals + gld * b}, lane, dt, n0, ne,
+                                                                Fb, tile, Db);
             __syncwarp();
         }
-        tile_eval<FORM, WIND, MODE, GOALS>(c, wsm + slot * SX_LEN, tile, tile_s, dt, k0, nk, lane, Fb, Gb, needF, needG, tsum,
-                                    !OP && t == 0 && (flow & FLOW_WAIT), tile_mis, OP ? tile : nullptr, Db, Zb);
+        tile_eval<FORM, WIND, MODE, GOALS, OP>(c, wsm + slot * SX_LEN, tile, tile_s, dt, k0, nk, lane, Fb, Gb, needF, needG,
+                                               tsum, !OP && t == 0 && (flow & FLOW_WAIT), tile_mis, OP ? tile : nullptr, Db,
+                                               Zb, OP ? goals + gld * b : nullptr);
         __syncwarp();
         const double sumT = warp_sum(tsum.sumT);
         const double sump = FORM == TOLCUDA_FORM_S10 || HVP ? warp_sum(tsum.sump) : 0.0;
@@ -1343,7 +1357,7 @@ __device__ __forceinline__ void fg_cta_body(const FgConst &c, int nrun, int per_
                 }
             }
             if (OP)
-                op_epilogue<FORM, MODE>(c, lane, dt, tT, n0, ne, Fb, Gb, tp, Db, Zb);
+                op_epilogue<FORM, MODE>(c, Goal<FORM, GOALS, true>{goals + gld * b}, lane, dt, tT, n0, ne, Fb, Gb, tp, Db, Zb);
             else
                 traj_epilogue<FORM>(c, Goal<FORM, GOALS>{wsm + slot * SX_LEN + GOAL_SX}, lane, dt, tT, tp, n0, ne, Fb,
                                            Gb, needF, mode_is_fonly(MODE) ? 0 : needG, dmax, dssq,
@@ -1357,19 +1371,20 @@ template <int FORM, int WIND, int MAXT, int MINB, int MODE, bool LOOP>
 __global__ void __launch_bounds__(MAXT, MINB)
 fg_cta_kernel(const __grid_constant__ FgConst c, int nrun, int per_arg, const double *__restrict__ x, long ldx,
                double *__restrict__ F, long ldF, double *__restrict__ G, long ldG, int needF, int needG, int flow,
-               double *__restrict__ S, long ldS) {
-    fg_cta_body<FORM, WIND, MAXT, MINB, MODE, LOOP, false>(c, nrun, per_arg, x, ldx, F, ldF, G, ldG, needF, needG, flow, S,
-                                                           ldS, nullptr);
+               double *__restrict__ S, long ldS, const double *__restrict__ goals, long gld) {
+    // goals, gld: the goal rows of the operator modes (the other modes use the context's FgConst immediates)
+    fg_cta_body<FORM, WIND, MAXT, MINB, MODE, LOOP, mode_is_op(MODE)>(c, nrun, per_arg, x, ldx, F, ldF, G, ldG, needF, needG,
+                                                                      flow, S, ldS, goals, gld);
 }
 
-// MODE_HVP: lam / w in the F / G places, then d and the optional z
+// MODE_HVP: lam / w in the F / G places, then d and the optional z, then the goal rows as in fg_cta_kernel
 template <int FORM, int WIND, int MAXT, int MINB, bool LOOP>
 __global__ void __launch_bounds__(MAXT, MINB)
 fg_cta_hvp_kernel(const __grid_constant__ FgConst c, int nrun, int per_arg, const double *__restrict__ x, long ldx,
                   double *__restrict__ lam, long ldl, double *__restrict__ w, long ldw, const double *__restrict__ d,
-                  long ldd, double *__restrict__ z, long ldz) {
-    fg_cta_body<FORM, WIND, MAXT, MINB, MODE_HVP, LOOP, false>(c, nrun, per_arg, x, ldx, lam, ldl, w, ldw, 1, 1, 0, nullptr, 0,
-                                                               nullptr, d, ldd, z, ldz);
+                  long ldd, double *__restrict__ z, long ldz, const double *__restrict__ goals, long gld) {
+    fg_cta_body<FORM, WIND, MAXT, MINB, MODE_HVP, LOOP, true>(c, nrun, per_arg, x, ldx, lam, ldl, w, ldw, 1, 1, 0, nullptr, 0,
+                                                              goals, gld, d, ldd, z, ldz);
 }
 
 template <int FORM, int WIND, int MAXT, int MINB, int MODE, bool LOOP>
@@ -1378,7 +1393,7 @@ fg_cta_goals_kernel(const __grid_constant__ FgConst c, int nrun, int per_arg, co
                     double *__restrict__ F, long ldF, double *__restrict__ G, long ldG, int needF, int needG, int flow,
                     double *__restrict__ S, long ldS, const double *__restrict__ goals) {
     fg_cta_body<FORM, WIND, MAXT, MINB, MODE, LOOP, true>(c, nrun, per_arg, x, ldx, F, ldF, G, ldG, needF, needG, flow, S,
-                                                          ldS, goals);
+                                                          ldS, goals, TOLCUDA_GOAL_LD);
 }
 
 // ---- kernel L: one CTA per trajectory of any length -------------------------------------------------------------
@@ -1389,14 +1404,15 @@ fg_cta_goals_kernel(const __grid_constant__ FgConst c, int nrun, int per_arg, co
 // trajectory with tolcuda_set_option(h, "kernel", 2)).  All warps of a CTA write the same G row, as in kernel A: the earlier
 // persistent-warp kernel (one whole trajectory per warp, 16 x 148 rows being written at a time) reached 0.82 of
 // the roofline on S10 ts=200 where kernel A reaches 0.98.
-// The body is shared by fg_long_kernel and fg_long_goals_kernel, as kernel A's.
+// The body is shared by fg_long_kernel and fg_long_goals_kernel, as kernel A's (the operator modes with GOALS).
 constexpr int LWARPS = 8;
 template <int FORM, int WIND, int MODE, bool GOALS>
 __device__ __forceinline__ void fg_long_body(const FgConst &c, const double *__restrict__ x, long ldx,
                                              double *__restrict__ F, long ldF, double *__restrict__ G, long ldG, int needF,
                                              int needG, int flow, double *__restrict__ S, long ldS,
-                                             const double *__restrict__ goals, const double *__restrict__ dm = nullptr,
-                                             long ldd = 0, double *__restrict__ zm = nullptr, long ldz = 0) {
+                                             const double *__restrict__ goals, long gld,
+                                             const double *__restrict__ dm = nullptr, long ldd = 0,
+                                             double *__restrict__ zm = nullptr, long ldz = 0) {
     pdl_release();
     constexpr bool SUMM = mode_has_summary(MODE);
     extern __shared__ __align__(16) double smem[];
@@ -1419,9 +1435,9 @@ __device__ __forceinline__ void fg_long_body(const FgConst &c, const double *__r
     double *Zb = HVP && zm ? zm + b * ldz : nullptr;
     slice_prefetch(wsm_s, xb + (size_t)PX * 32 * warp, 1 + PX * (min(32, ts - 32 * warp) + 1), lane);
     // S10: the goal values go into both slice buffers with the first slice; the later slices leave them alone
-    if (GOALS && FORM == TOLCUDA_FORM_S10) {
-        goal_prefetch<FORM>(wsm_s, goals + TOLCUDA_GOAL_LD * b, lane);
-        goal_prefetch<FORM>(wsm_s + 8 * SX_LEN, goals + TOLCUDA_GOAL_LD * b, lane);
+    if (GOALS && !OP && FORM == TOLCUDA_FORM_S10) {
+        goal_prefetch<FORM>(wsm_s, goals + gld * b, lane);
+        goal_prefetch<FORM>(wsm_s + 8 * SX_LEN, goals + gld * b, lane);
     }
     cp_async_commit();
     const double dt = __ldg(xb);
@@ -1449,12 +1465,13 @@ __device__ __forceinline__ void fg_long_body(const FgConst &c, const double *__r
         __syncwarp();
         TileSums tsum;
         if ((MODE == MODE_VJP || HVP) && (j == 0 || j == nt - 1)) {  // the tiles that own node 0 / node ts (warp-uniform)
-            op_aux<FORM, std::conditional_t<HVP, Dual, double>>(c, lane, dt, n0, ne, Fb, tile, Db);
+            op_aux<FORM, std::conditional_t<HVP, Dual, double>>(c, Goal<FORM, GOALS, true>{GOALS ? goals + gld * b : nullptr},
+                                                                lane, dt, n0, ne, Fb, tile, Db);
             __syncwarp();
         }
-        tile_eval<FORM, WIND, MODE, GOALS>(c, wsm + slot * SX_LEN, tile, tile_s, dt, 32 * j, min(32, ts - 32 * j), lane, Fb, Gb,
-                                    needF, needG, tsum, !OP && j == warp && (flow & FLOW_WAIT), tile_mis, OP ? tile : nullptr,
-                                    Db, Zb);
+        tile_eval<FORM, WIND, MODE, GOALS, OP>(c, wsm + slot * SX_LEN, tile, tile_s, dt, 32 * j, min(32, ts - 32 * j), lane,
+                                               Fb, Gb, needF, needG, tsum, !OP && j == warp && (flow & FLOW_WAIT), tile_mis,
+                                               OP ? tile : nullptr, Db, Zb, OP ? goals + gld * b : nullptr);
         __syncwarp();
         accT += tsum.sumT;
         accp += tsum.sump;
@@ -1491,9 +1508,10 @@ __device__ __forceinline__ void fg_long_body(const FgConst &c, const double *__r
         }
     }
     if (OP)
-        op_epilogue<FORM, MODE>(c, lane, dt, tT, n0, ne, Fb, Gb, tp, Db, Zb);
+        op_epilogue<FORM, MODE>(c, Goal<FORM, GOALS, true>{GOALS ? goals + gld * b : nullptr}, lane, dt, tT, n0, ne, Fb, Gb,
+                                tp, Db, Zb);
     else
-        traj_epilogue<FORM>(c, Goal<FORM, GOALS, true>{GOALS ? goals + TOLCUDA_GOAL_LD * b : nullptr}, lane, dt, tT, tp, n0, ne, Fb, Gb, needF,
+        traj_epilogue<FORM>(c, Goal<FORM, GOALS, true>{GOALS ? goals + gld * b : nullptr}, lane, dt, tT, tp, n0, ne, Fb, Gb, needF,
                                    mode_is_fonly(MODE) ? 0 : needG, dmax, dssq, SUMM ? S + b * ldS : nullptr,
                                    MODE == MODE_COMPACT ? NVAR : REC);
 }
@@ -1502,8 +1520,9 @@ template <int FORM, int WIND, int MODE>
 __global__ void __launch_bounds__(LWARPS * 32, 2)
 fg_long_kernel(const __grid_constant__ FgConst c, const double *__restrict__ x, long ldx,
                double *__restrict__ F, long ldF, double *__restrict__ G, long ldG, int needF, int needG, int flow,
-               double *__restrict__ S, long ldS) {
-    fg_long_body<FORM, WIND, MODE, false>(c, x, ldx, F, ldF, G, ldG, needF, needG, flow, S, ldS, nullptr);
+               double *__restrict__ S, long ldS, const double *__restrict__ goals, long gld) {
+    // goals, gld: as in fg_cta_kernel
+    fg_long_body<FORM, WIND, MODE, mode_is_op(MODE)>(c, x, ldx, F, ldF, G, ldG, needF, needG, flow, S, ldS, goals, gld);
 }
 
 // MODE_HVP, as fg_cta_hvp_kernel
@@ -1512,8 +1531,8 @@ template <int FORM, int WIND>
 __global__ void __launch_bounds__(LWARPS * 32, HVP_LMINB)
 fg_long_hvp_kernel(const __grid_constant__ FgConst c, const double *__restrict__ x, long ldx, double *__restrict__ lam,
                    long ldl, double *__restrict__ w, long ldw, const double *__restrict__ d, long ldd,
-                   double *__restrict__ z, long ldz) {
-    fg_long_body<FORM, WIND, MODE_HVP, false>(c, x, ldx, lam, ldl, w, ldw, 1, 1, 0, nullptr, 0, nullptr, d, ldd, z, ldz);
+                   double *__restrict__ z, long ldz, const double *__restrict__ goals, long gld) {
+    fg_long_body<FORM, WIND, MODE_HVP, true>(c, x, ldx, lam, ldl, w, ldw, 1, 1, 0, nullptr, 0, goals, gld, d, ldd, z, ldz);
 }
 
 template <int FORM, int WIND, int MODE>
@@ -1521,7 +1540,7 @@ __global__ void __launch_bounds__(LWARPS * 32, 2)
 fg_long_goals_kernel(const __grid_constant__ FgConst c, const double *__restrict__ x, long ldx,
                      double *__restrict__ F, long ldF, double *__restrict__ G, long ldG, int needF, int needG, int flow,
                      double *__restrict__ S, long ldS, const double *__restrict__ goals) {
-    fg_long_body<FORM, WIND, MODE, true>(c, x, ldx, F, ldF, G, ldG, needF, needG, flow, S, ldS, goals);
+    fg_long_body<FORM, WIND, MODE, true>(c, x, ldx, F, ldF, G, ldG, needF, needG, flow, S, ldS, goals, TOLCUDA_GOAL_LD);
 }
 
 // one launch, optionally as a programmatic dependent of the launch before it on the stream (FgLaunch::pdl)
@@ -1565,13 +1584,13 @@ cudaError_t launch_cta_as(const FgLaunch &L, const int per, const int nsingle) {
     const int grid = LOOP ? nrun + nsingle : L.B;
     if constexpr (MODE == MODE_HVP)
         return launch_kernel(kern, grid, nthr, smem, L, *L.c, nrun, per, L.x, L.ldx, L.F, L.ldF, L.G, L.ldG, L.D, L.ldD,
-                             L.Z, L.ldZ);
+                             L.Z, L.ldZ, L.goals, L.goal_ld);
     else if constexpr (GOALS)
         return launch_kernel(kern, grid, nthr, smem, L, *L.c, nrun, per, L.x, L.ldx, L.F, L.ldF, L.G, L.ldG, L.needF,
                              L.needG, L.pdl == 1 ? FLOW_WAIT : 0, L.S, L.ldS, L.goals);
     else
         return launch_kernel(kern, grid, nthr, smem, L, *L.c, nrun, per, L.x, L.ldx, L.F, L.ldF, L.G, L.ldG, L.needF,
-                             L.needG, L.pdl == 1 ? FLOW_WAIT : 0, L.S, L.ldS);
+                             L.needG, L.pdl == 1 ? FLOW_WAIT : 0, L.S, L.ldS, L.goals, L.goal_ld);
 }
 
 // Runs of `per` trajectories per CTA pay off once the grid is many waves deep (the x load and the CTA launch
@@ -1605,13 +1624,14 @@ cudaError_t launch_long(const FgLaunch &L) {
     const size_t smem = sizeof(double) * (size_t)(nthr / 32) * WARP_SMEM_B;
     if (cudaError_t e = reserve_smem<kern>(L, smem)) return e;
     if constexpr (MODE == MODE_HVP)
-        return launch_kernel(kern, L.B, nthr, smem, L, *L.c, L.x, L.ldx, L.F, L.ldF, L.G, L.ldG, L.D, L.ldD, L.Z, L.ldZ);
+        return launch_kernel(kern, L.B, nthr, smem, L, *L.c, L.x, L.ldx, L.F, L.ldF, L.G, L.ldG, L.D, L.ldD, L.Z, L.ldZ,
+                             L.goals, L.goal_ld);
     else if constexpr (GOALS)
         return launch_kernel(kern, L.B, nthr, smem, L, *L.c, L.x, L.ldx, L.F, L.ldF, L.G, L.ldG, L.needF, L.needG,
                              L.pdl == 1 ? FLOW_WAIT : 0, L.S, L.ldS, L.goals);
     else
         return launch_kernel(kern, L.B, nthr, smem, L, *L.c, L.x, L.ldx, L.F, L.ldF, L.G, L.ldG, L.needF, L.needG,
-                             L.pdl == 1 ? FLOW_WAIT : 0, L.S, L.ldS);
+                             L.pdl == 1 ? FLOW_WAIT : 0, L.S, L.ldS, L.goals, L.goal_ld);
 }
 
 
@@ -1637,7 +1657,7 @@ cudaError_t launch_sel(const FgLaunch &L) {
 }
 
 // the per-trajectory summary is a separate instantiation so that plain F/G launches pay nothing for it; so is a
-// goal table (GOALS), and the matrix-free modes have no instances with one
+// goal table (GOALS).  The matrix-free modes have no goal instances: they always read their goal from L.goals
 template <int FORM, int WIND, bool GOALS>
 cudaError_t launch_flavour(const FgLaunch &L) {
     if (L.compact) return launch_sel<FORM, WIND, MODE_COMPACT, GOALS>(L);
@@ -1648,7 +1668,6 @@ cudaError_t launch_flavour(const FgLaunch &L) {
 
 template <int FORM, int WIND>
 cudaError_t launch_any(const FgLaunch &L) {
-    if (L.op && L.goals) return cudaErrorInvalidValue;
     if (L.op == 1) return launch_sel<FORM, WIND, MODE_JVP, false>(L);
     if (L.op == 2) return launch_sel<FORM, WIND, MODE_VJP, false>(L);
     if (L.op == 3) return launch_sel<FORM, WIND, MODE_HVP, false>(L);
@@ -1659,7 +1678,7 @@ cudaError_t launch_any(const FgLaunch &L) {
 
 cudaError_t fg_launch(const FgLaunch &L) {
     if (L.B <= 0) return cudaSuccess;
-    if (!L.c || L.c->ts < 1) return cudaErrorInvalidValue;
+    if (!L.c || L.c->ts < 1 || (L.op && !L.goals)) return cudaErrorInvalidValue;
     if (L.c->form == TOLCUDA_FORM_S10) {
         if (L.c->wind == 1) return launch_any<TOLCUDA_FORM_S10, 1>(L);
         if (L.c->wind == 0) return launch_any<TOLCUDA_FORM_S10, 0>(L);

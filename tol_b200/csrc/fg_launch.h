@@ -37,8 +37,10 @@ struct FgLaunch {
     int pdl;       // 0: ordinary launch; 1: programmatic dependent launch, the kernel waits for the preceding launch on
                    // the stream before its first store; 2: the same without the wait (outputs disjoint from the
                    // preceding launch's reads and writes).  Never set for op != 0 (d / lambda are read early).
-    const double *goals;  // NULL: every trajectory has the context's goal; else trajectory b's goal is the row
-                          // goals + TOLCUDA_GOAL_LD*b of a device goal table (op == 0 only)
+    const double *goals;  // op == 0: NULL, every trajectory has the context's goal (FgConst); else trajectory b's goal
+                          // is the row goals + TOLCUDA_GOAL_LD*b of a device goal table.  op != 0: never NULL,
+                          // trajectory b's goal is the row goals + goal_ld*b
+    long goal_ld;         // op != 0: TOLCUDA_GOAL_LD for a goal table, 0 for the context's own goal row
     int sm_count;  // SMs of the device
     int device;    // CUDA device ordinal the launch goes to (the current device)
     cudaStream_t stream;

@@ -90,6 +90,7 @@ struct tolcuda_ctx {
     int *d_perm = nullptr;     // CSC position -> coordinate-order position, uploaded at first use
     double *d_goals = nullptr;  // goal table (tolcuda_set_goals): ngoals rows of TOLCUDA_GOAL_LD doubles (goal_row)
     long ngoals = 0;
+    double *d_goal = nullptr;   // the context's goal as one such row: the matrix-free products read it with row stride 0
     std::string dump_dir;      // DEFINEGusrfg_: the reference's per-call dump files go here (empty: none)
     bool dump_warned = false;
 };
@@ -113,13 +114,15 @@ void goal_row(const double *goal, double row[TOLCUDA_GOAL_LD]) {
     for (int i = 5; i < TOLCUDA_GOAL_LD; i++) row[i] = 0.0;
 }
 
-// goals: NULL, or the device goal-table row of the launch's first trajectory
+// goals: NULL, or the device goal-table row of the launch's first trajectory.  The matrix-free products (op != 0) read
+// a NULL goals as the context's goal row, for every trajectory.
 int launch(tolcuda_ctx *h, cudaStream_t st, int B, const double *x, long ldx, double *F, long ldF,
            double *G, long ldG, int needF, int needG, double *S = nullptr, long ldS = 0, int compact = 0, int op = 0,
            int pdl = 0, const double *goals = nullptr, const double *D = nullptr, long ldD = 0, double *Z = nullptr,
            long ldZ = 0) {
     FgLaunch L{};
-    L.goals = goals;
+    L.goals = goals, L.goal_ld = TOLCUDA_GOAL_LD;
+    if (op && !goals) L.goals = h->d_goal, L.goal_ld = 0;
     L.D = D, L.ldD = ldD, L.Z = Z, L.ldZ = ldZ;
     L.S = S, L.ldS = ldS;
     L.compact = compact;
@@ -397,6 +400,10 @@ int tolcuda_create(const tolcuda_config *cfg, tolcuda_handle *out) {
         if (e != cudaSuccess) { rc = cuda_fail(e, "cudaMallocHost"); break; }
         e = cudaMalloc(&h->d_one, bytes);
         if (e != cudaSuccess) { rc = cuda_fail(e, "cudaMalloc"); break; }
+        e = cudaMalloc(&h->d_goal, sizeof(grow));
+        if (e != cudaSuccess) { rc = cuda_fail(e, "cudaMalloc"); break; }
+        e = cudaMemcpy(h->d_goal, grow, sizeof(grow), cudaMemcpyHostToDevice);
+        if (e != cudaSuccess) { rc = cuda_fail(e, "cudaMemcpy"); break; }
     } while (0);
     if (rc) {
         tolcuda_destroy(h);
@@ -502,6 +509,7 @@ int tolcuda_destroy(tolcuda_handle h) {
     if (h->d_grid) cudaFree(h->d_grid);
     if (h->d_perm) cudaFree(h->d_perm);
     if (h->d_goals) cudaFree(h->d_goals);
+    if (h->d_goal) cudaFree(h->d_goal);
     if (h->own_stream) cudaStreamDestroy(h->own_stream);
     delete h;
     return 0;
@@ -796,22 +804,30 @@ int tolcuda_set_goals(tolcuda_handle h, long count, const double *goal, long ldg
     return 0;
 }
 
-int tolcuda_eval_batch_goals(tolcuda_handle h, long row0, int B, const double *x, long ldx, double *F, long ldF,
-                             double *G, long ldG, double *summary, long lds, int flags) {
+// the device row of goal row0 of the context's table, for a call of B trajectories with goal rows row0 .. row0 + B - 1;
+// NULL (error set) for a null handle, no table, or rows outside the table
+static const double *goal_rows(tolcuda_handle h, long row0, int B, const char *who) {
     if (!h) {
-        set_error("tolcuda_eval_batch_goals: null handle");
-        return TOLCUDA_EINVAL;
+        set_error(std::string(who) + ": null handle");
+        return nullptr;
     }
     if (!h->d_goals) {
-        set_error("tolcuda_eval_batch_goals: no goal table (tolcuda_set_goals)");
-        return TOLCUDA_EINVAL;
+        set_error(std::string(who) + ": no goal table (tolcuda_set_goals)");
+        return nullptr;
     }
     if (row0 < 0 || B < 0 || row0 + B > h->ngoals) {
-        set_error("tolcuda_eval_batch_goals: rows [" + std::to_string(row0) + ", " + std::to_string(row0 + B) +
+        set_error(std::string(who) + ": rows [" + std::to_string(row0) + ", " + std::to_string(row0 + B) +
                   ") outside the goal table's " + std::to_string(h->ngoals) + " rows");
-        return TOLCUDA_EINVAL;
+        return nullptr;
     }
-    return eval_batch(h, B, x, ldx, F, ldF, G, ldG, summary, lds, flags, h->d_goals + (size_t)TOLCUDA_GOAL_LD * row0);
+    return h->d_goals + (size_t)TOLCUDA_GOAL_LD * row0;
+}
+
+int tolcuda_eval_batch_goals(tolcuda_handle h, long row0, int B, const double *x, long ldx, double *F, long ldF,
+                             double *G, long ldG, double *summary, long lds, int flags) {
+    const double *goals = goal_rows(h, row0, B, "tolcuda_eval_batch_goals");
+    if (!goals) return TOLCUDA_EINVAL;
+    return eval_batch(h, B, x, ldx, F, ldF, G, ldG, summary, lds, flags, goals);
 }
 
 long tolcuda_compact_len(int formulation, int ts) {
@@ -849,9 +865,10 @@ int tolcuda_expand_compact_g_device(tolcuda_handle h, long B, const double *Gc, 
     return 0;
 }
 
-// y = J(x) d and z = J(x)^T lambda without materialising G (fg_kernels.cu, MODE_JVP / MODE_VJP)
+// y = J(x) d and z = J(x)^T lambda without materialising G (fg_kernels.cu, MODE_JVP / MODE_VJP).  goals: NULL (the
+// context's goal), or the goal-table row of trajectory 0
 static int jac_op(tolcuda_handle h, int op, int B, const double *x, long ldx, const double *in, long ldin, long len_in,
-                  double *out, long ldout, long len_out, int flags, const char *who) {
+                  double *out, long ldout, long len_out, int flags, const char *who, const double *goals = nullptr) {
     if (!h || B < 0) return TOLCUDA_EINVAL;
     if (B == 0) return 0;
     const FgConst &c = h->c;
@@ -867,7 +884,7 @@ static int jac_op(tolcuda_handle h, int op, int B, const double *x, long ldx, co
     // op 1: the F pointer receives y, the G pointer holds d; op 2: the F pointer holds lambda, the G pointer receives z
     double *Fp = op == 1 ? out : const_cast<double *>(in), *Gp = op == 1 ? const_cast<double *>(in) : out;
     const long ldFp = op == 1 ? ldout : ldin, ldGp = op == 1 ? ldin : ldout;
-    int rc = launch(h, h->stream, B, x, ldx, Fp, ldFp, Gp, ldGp, 1, 1, nullptr, 0, 0, op);
+    int rc = launch(h, h->stream, B, x, ldx, Fp, ldFp, Gp, ldGp, 1, 1, nullptr, 0, 0, op, 0, goals);
     if (rc) return rc;
     if (!(flags & TOLCUDA_NO_SYNC)) CU(cudaStreamSynchronize(h->stream));
     return 0;
@@ -883,26 +900,53 @@ int tolcuda_jac_tvec(tolcuda_handle h, int B, const double *x, long ldx, const d
     return jac_op(h, 2, B, x, ldx, lambda, ldl, h ? h->c.neF : 0, z, ldz, h ? h->c.n : 0, flags, "tolcuda_jac_tvec");
 }
 
-// w = D_x[J(x)^T lambda] d and optionally z = J(x)^T lambda (fg_kernels.cu, MODE_HVP)
-int tolcuda_lag_hess_vec(tolcuda_handle h, int B, const double *x, long ldx, const double *lambda, long ldl,
-                         const double *d, long ldd, double *w, long ldw, double *z, long ldz, int flags) {
+int tolcuda_jac_vec_goals(tolcuda_handle h, long row0, int B, const double *x, long ldx, const double *d, long ldd,
+                          double *y, long ldy, int flags) {
+    const double *goals = goal_rows(h, row0, B, "tolcuda_jac_vec_goals");
+    if (!goals) return TOLCUDA_EINVAL;
+    return jac_op(h, 1, B, x, ldx, d, ldd, h->c.n, y, ldy, h->c.neF, flags, "tolcuda_jac_vec_goals", goals);
+}
+
+int tolcuda_jac_tvec_goals(tolcuda_handle h, long row0, int B, const double *x, long ldx, const double *lambda, long ldl,
+                           double *z, long ldz, int flags) {
+    const double *goals = goal_rows(h, row0, B, "tolcuda_jac_tvec_goals");
+    if (!goals) return TOLCUDA_EINVAL;
+    return jac_op(h, 2, B, x, ldx, lambda, ldl, h->c.neF, z, ldz, h->c.n, flags, "tolcuda_jac_tvec_goals", goals);
+}
+
+// w = D_x[J(x)^T lambda] d and optionally z = J(x)^T lambda (fg_kernels.cu, MODE_HVP); goals as in jac_op
+static int lag_hess(tolcuda_handle h, int B, const double *x, long ldx, const double *lambda, long ldl, const double *d,
+                    long ldd, double *w, long ldw, double *z, long ldz, int flags, const char *who,
+                    const double *goals = nullptr) {
     if (!h || B < 0) return TOLCUDA_EINVAL;
     if (B == 0) return 0;
     const FgConst &c = h->c;
     if (!x || !lambda || !d || !w || ldx < c.n || ldl < c.neF || ldd < c.n || ldw < c.n || (z && ldz < c.n)) {
-        set_error("tolcuda_lag_hess_vec: null pointer or leading dimension shorter than the row");
+        set_error(std::string(who) + ": null pointer or leading dimension shorter than the row");
         return TOLCUDA_EINVAL;
     }
     if (flags & TOLCUDA_HOST_PTRS) {
-        set_error("tolcuda_lag_hess_vec: device pointers only");
+        set_error(std::string(who) + ": device pointers only");
         return TOLCUDA_EUNSUPPORTED;
     }
     CU(cudaSetDevice(h->cfg.device));
-    int rc = launch(h, h->stream, B, x, ldx, const_cast<double *>(lambda), ldl, w, ldw, 1, 1, nullptr, 0, 0, 3, 0, nullptr,
+    int rc = launch(h, h->stream, B, x, ldx, const_cast<double *>(lambda), ldl, w, ldw, 1, 1, nullptr, 0, 0, 3, 0, goals,
                     d, ldd, z, z ? ldz : 0);
     if (rc) return rc;
     if (!(flags & TOLCUDA_NO_SYNC)) CU(cudaStreamSynchronize(h->stream));
     return 0;
+}
+
+int tolcuda_lag_hess_vec(tolcuda_handle h, int B, const double *x, long ldx, const double *lambda, long ldl,
+                         const double *d, long ldd, double *w, long ldw, double *z, long ldz, int flags) {
+    return lag_hess(h, B, x, ldx, lambda, ldl, d, ldd, w, ldw, z, ldz, flags, "tolcuda_lag_hess_vec");
+}
+
+int tolcuda_lag_hess_vec_goals(tolcuda_handle h, long row0, int B, const double *x, long ldx, const double *lambda,
+                               long ldl, const double *d, long ldd, double *w, long ldw, double *z, long ldz, int flags) {
+    const double *goals = goal_rows(h, row0, B, "tolcuda_lag_hess_vec_goals");
+    if (!goals) return TOLCUDA_EINVAL;
+    return lag_hess(h, B, x, ldx, lambda, ldl, d, ldd, w, ldw, z, ldz, flags, "tolcuda_lag_hess_vec_goals", goals);
 }
 
 int tolcuda_problem_pattern_csc(int formulation, int ts, int *colptr, int *rowidx, int *perm) {

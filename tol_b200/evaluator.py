@@ -338,28 +338,41 @@ class Evaluator:
         _l.check(self.L.tolcuda_repack_csc_device(self.h, G.shape[0], G.data_ptr(), G.stride(0), Gcsc.data_ptr(),
                                                   Gcsc.stride(0), 0 if sync else NO_SYNC))
 
-    def jac_vec(self, X, D, Y, sync=True):
+    def jac_vec(self, X, D, Y, sync=True, row0=None):
         """tolcuda_jac_vec: Y[b] = J(X[b]) D[b] without materialising G (torch CUDA tensors [B, >= n], [B, >= n],
-        [B, >= neF])"""
+        [B, >= neF]).  row0: None for the context's goal, else tolcuda_jac_vec_goals with goal row row0 + b of the
+        table (set_goals) for row b"""
         self._follow_torch(X)
-        _l.check(self.L.tolcuda_jac_vec(self.h, X.shape[0], X.data_ptr(), X.stride(0), D.data_ptr(), D.stride(0),
-                                        Y.data_ptr(), Y.stride(0), 0 if sync else NO_SYNC))
+        args = (X.shape[0], X.data_ptr(), X.stride(0), D.data_ptr(), D.stride(0), Y.data_ptr(), Y.stride(0),
+                0 if sync else NO_SYNC)
+        if row0 is None:
+            _l.check(self.L.tolcuda_jac_vec(self.h, *args))
+        else:
+            _l.check(self.L.tolcuda_jac_vec_goals(self.h, int(row0), *args))
 
-    def jac_tvec(self, X, Lam, Z, sync=True):
-        """tolcuda_jac_tvec: Z[b] = J(X[b])^T Lam[b] (torch CUDA tensors [B, >= n], [B, >= neF], [B, >= n])"""
+    def jac_tvec(self, X, Lam, Z, sync=True, row0=None):
+        """tolcuda_jac_tvec: Z[b] = J(X[b])^T Lam[b] (torch CUDA tensors [B, >= n], [B, >= neF], [B, >= n]).  row0: as
+        in jac_vec (tolcuda_jac_tvec_goals)"""
         self._follow_torch(X)
-        _l.check(self.L.tolcuda_jac_tvec(self.h, X.shape[0], X.data_ptr(), X.stride(0), Lam.data_ptr(), Lam.stride(0),
-                                         Z.data_ptr(), Z.stride(0), 0 if sync else NO_SYNC))
+        args = (X.shape[0], X.data_ptr(), X.stride(0), Lam.data_ptr(), Lam.stride(0), Z.data_ptr(), Z.stride(0),
+                0 if sync else NO_SYNC)
+        if row0 is None:
+            _l.check(self.L.tolcuda_jac_tvec(self.h, *args))
+        else:
+            _l.check(self.L.tolcuda_jac_tvec_goals(self.h, int(row0), *args))
 
-    def lag_hess_vec(self, X, Lam, D, W, Z=None, sync=True):
+    def lag_hess_vec(self, X, Lam, D, W, Z=None, sync=True, row0=None):
         """tolcuda_lag_hess_vec: W[b] = D_x[J(X[b])^T Lam[b]] D[b], the Hessian of the Lagrangian Lam[b]^T F times D[b],
         and, if Z is given, Z[b] = J(X[b])^T Lam[b] (torch CUDA tensors [B, >= n], [B, >= neF], [B, >= n], [B, >= n],
-        [B, >= n])"""
+        [B, >= n]).  row0: as in jac_vec (tolcuda_lag_hess_vec_goals)"""
         self._follow_torch(X)
-        _l.check(self.L.tolcuda_lag_hess_vec(self.h, X.shape[0], X.data_ptr(), X.stride(0), Lam.data_ptr(), Lam.stride(0),
-                                             D.data_ptr(), D.stride(0), W.data_ptr(), W.stride(0),
-                                             None if Z is None else Z.data_ptr(), 0 if Z is None else Z.stride(0),
-                                             0 if sync else NO_SYNC))
+        args = (X.shape[0], X.data_ptr(), X.stride(0), Lam.data_ptr(), Lam.stride(0), D.data_ptr(), D.stride(0),
+                W.data_ptr(), W.stride(0), None if Z is None else Z.data_ptr(), 0 if Z is None else Z.stride(0),
+                0 if sync else NO_SYNC)
+        if row0 is None:
+            _l.check(self.L.tolcuda_lag_hess_vec(self.h, *args))
+        else:
+            _l.check(self.L.tolcuda_lag_hess_vec_goals(self.h, int(row0), *args))
 
     def summary_host(self, X, needF=False, needG=False):
         """tolcuda_eval_batch_summary with host arrays: [B, 4] = objective, max|defect|, max boundary

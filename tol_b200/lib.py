@@ -67,6 +67,10 @@ def load():
     L.tolcuda_jac_tvec.argtypes = [vp, C.c_int, vp, C.c_long, vp, C.c_long, vp, C.c_long, C.c_int]
     L.tolcuda_lag_hess_vec.argtypes = [vp, C.c_int, vp, C.c_long, vp, C.c_long, vp, C.c_long, vp, C.c_long, vp,
                                        C.c_long, C.c_int]
+    L.tolcuda_jac_vec_goals.argtypes = [vp, C.c_long, C.c_int, vp, C.c_long, vp, C.c_long, vp, C.c_long, C.c_int]
+    L.tolcuda_jac_tvec_goals.argtypes = [vp, C.c_long, C.c_int, vp, C.c_long, vp, C.c_long, vp, C.c_long, C.c_int]
+    L.tolcuda_lag_hess_vec_goals.argtypes = [vp, C.c_long, C.c_int, vp, C.c_long, vp, C.c_long, vp, C.c_long, vp,
+                                             C.c_long, vp, C.c_long, C.c_int]
     L.tolcuda_host_alloc.argtypes = [C.c_size_t, C.POINTER(vp)]
     L.tolcuda_host_free.argtypes = [vp]
     L.tolcuda_device_count.argtypes = [ip]

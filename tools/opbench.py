@@ -1,8 +1,10 @@
 #!/usr/bin/env python
 """Matrix-free Jacobian products (tolcuda_jac_vec / tolcuda_jac_tvec) next to the F+G evaluation they replace
 when G itself is not wanted, and the Hessian-of-the-Lagrangian product (tolcuda_lag_hess_vec) next to the central
-difference of two tolcuda_jac_tvec launches it replaces: device-resident, CUDA events on the launching stream.  The
-first line names the card and its power limit, read in the same run.
+difference of two tolcuda_jac_tvec launches it replaces: device-resident, CUDA events on the launching stream.  Then
+the goal-table arm: y, z and w with a table of B distinct goals (tolcuda_*_goals) against the same products with the
+context's goal, and w for 256 goals x 64 trajectories as one tolcuda_lag_hess_vec_goals launch against 256 per-goal
+contexts launched one after another.  The first line names the card and its power limit, read in the same run.
 
     python tools/opbench.py [--workload S10_tempest_ts200] [--batch 65536] [--steps 20]"""
 import argparse
@@ -82,4 +84,33 @@ for label, fn, by in (
     ms = timed(fn)
     print(json.dumps({"workload": args.workload, "B": B, "op": label, "ms": ms, "node_evals_per_s": B * ts / (ms * 1e-3),
                       "algorithmic_GB": by / 1e9, "GBps": by / ms / 1e6, "frac_of_6544": by / ms / 1e6 / 6544.0}))
+
+# goal-table arm: every trajectory its own goal, against the context's goal (the rows above)
+mission = str(g["mission"])
+ev.set_goals(T.synth.goals(mission, 0, B))
+for label, fn in (("y = J d, goal table", lambda: ev.jac_vec(Xd, D, Y, sync=False, row0=0)),
+                  ("z = J^T lambda, goal table", lambda: ev.jac_tvec(Xd, Lam, Z, sync=False, row0=0)),
+                  ("w = H d, goal table", lambda: ev.lag_hess_vec(Xd, Lam, D, W, sync=False, row0=0))):
+    print(json.dumps({"workload": args.workload, "B": B, "op": label, "goals": B, "ms": timed(fn)}))
+
+# 256 missions x 64 trajectories: one launch with a goal table against one context (and one launch) per mission
+K, R = 256, 64
+if B >= K * R:
+    goals = T.synth.goals(mission, 0, K)
+    ev.set_goals(np.repeat(goals, R, axis=0))
+    Xs, Ls, Ds, Ws = Xd[:K * R], Lam[:K * R], D[:K * R], W[:K * R]
+    print(json.dumps({"workload": args.workload, "op": "w = H d, one launch, %d goals x %d" % (K, R),
+                      "ms": timed(lambda: ev.lag_hess_vec(Xs, Ls, Ds, Ws, sync=False, row0=0))}))
+    ctxs = [T.Evaluator(mission, ts, g["ac"], g["gn"], goals[k], int(g["wind_model"])) for k in range(K)]
+    for e in ctxs:
+        e.set_stream(st.cuda_stream)
+
+    def per_goal_contexts():
+        for k, e in enumerate(ctxs):
+            s = slice(k * R, (k + 1) * R)
+            e.lag_hess_vec(Xs[s], Ls[s], Ds[s], Ws[s], sync=False)
+    print(json.dumps({"workload": args.workload, "op": "w = H d, %d per-goal contexts x %d" % (K, R),
+                      "ms": timed(per_goal_contexts)}))
+    for e in ctxs:
+        e.close()
 ev.close()
